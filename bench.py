@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- MCTS simulations/s of the self-play hot path on N B200s (one process per GPU).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--config gomoku|connect4|gumbel|tictactoe]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--config gomoku|connect4|gumbel|tictactoe] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N --steps K --warmup W
     python bench.py --impl reference ...     # CPU arm: the oracle port of the reference path on the host cores
 
@@ -146,7 +146,7 @@ class SelfPlayBench:
     """Drives the engine the way Self_Play.play does (two PUCT trees per game, the tree of the side to move
     searches, both are re-rooted after the move; one fresh Gumbel tree per move)."""
 
-    def __init__(self, cfg, n_games, device, noise=True, pool_fraction=1.0, eval_cache=0):
+    def __init__(self, cfg, n_games, device, noise=True, pool_fraction=1.0, eval_cache=0, keep_roots=False):
         from grok_alpha_zero_b200 import netspec
         from grok_alpha_zero_b200.engine import Engine
         from grok_alpha_zero_b200.net import Net
@@ -183,6 +183,9 @@ class SelfPlayBench:
         self.next_player = np.full(n_games, -1, np.int32)
         self.alive = np.ones(n_games, bool)
         self.launches = 0
+        # keep_roots: advance_move keeps the root statistics of the search it finishes (value sums included) in last_roots,
+        # so that what a search handed its caller can still be read after the trees were re-rooted
+        self.keep_roots, self.last_roots = keep_roots, None
         self.per_round_launches = 3 + 1 + self.net.n_launches  # counter reset, select, expand + chunk count + network kernels
         if eval_cache > 0:
             self.per_round_launches += 2                       # cache look-up and fill passes
@@ -228,6 +231,7 @@ class SelfPlayBench:
     def rounds(self, n, sync=False):
         self.eng.rounds_net(n, sync=sync)
         self.launches += n * self.per_round_launches
+        self.last_roots = None
 
     def run_finished(self):
         return self.eng.remaining() == 0
@@ -235,7 +239,9 @@ class SelfPlayBench:
     def advance_move(self):
         """root stats -> tau=0 move -> do_action/check_win -> prune_tree on both trees -> next run"""
         e = self.eng
-        _, _, info = e.root_dense(want_values=False)
+        vis, val, info = e.root_dense(want_values=self.keep_roots)
+        if self.keep_roots:
+            self.last_roots = (vis, val, info)
         info = info.reshape(self.n_games, self.tpg, 4)
         run_tree = 0 if self.gumbel else (self.next_player > 0).astype(int)
         sel = info[np.arange(self.n_games), run_tree]
@@ -267,6 +273,29 @@ class SelfPlayBench:
 
     def total_sims(self):
         return self.sims_done + self.sims_in_flight()
+
+
+DUMP_LIMIT_BYTES = 64 * 10 ** 6 - 4096     # 64 MB less room for the .npy headers
+
+
+def dump_outputs(sb, folder):
+    """Root statistics of every tree after the last timed search round (gaz_root_dense: visit counts and value sums by action
+    id, per-tree root visits / tau=0 move / iterations / evaluations), written as float32 / float64 .npy files so that two
+    builds can be compared output for output.  If the timed region ended with a move transition, they are the statistics
+    that move was chosen from, not those of the re-rooted trees.  Above 64 MB a fixed seeded sample of trees is written,
+    with its tree indices."""
+    vis, val, info = sb.last_roots if sb.last_roots is not None else sb.eng.root_dense(want_values=True)
+    out = dict(root_visits=vis.astype(np.float32), root_value_sums=val.astype(np.float32), root_info=info.astype(np.float64))
+    n_trees = vis.shape[0]
+    row_bytes = sum(a[0].nbytes for a in out.values())
+    keep = min(n_trees, (DUMP_LIMIT_BYTES - 8 * n_trees) // row_bytes)
+    if keep < n_trees:
+        rows = np.sort(np.random.default_rng(0).choice(n_trees, keep, replace=False))
+        out = {k: a[rows] for k, a in out.items()}
+        out["tree_index"] = rows.astype(np.float64)
+    os.makedirs(folder, exist_ok=True)
+    for k, a in out.items():
+        np.save(os.path.join(folder, k + ".npy"), a)
 
 
 def dominant_kernel_stats(sb, leaves_per_launch, peaks):
@@ -439,7 +468,7 @@ def run_moves(args, cfg, sb, timed_moves, barrier, world, rank, local, n_games):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=40)
+    ap.add_argument("--steps", type=int, default=None, help="timed search rounds (default 40)")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="ours")
     ap.add_argument("--config", default="gomoku", choices=sorted(CONFIGS))
@@ -449,7 +478,7 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--moves", type=int, default=0,
                     help="time M WHOLE moves per game from the start position (search, move choice, do_action, prune_tree / "
-                         "re-rooting of both trees) instead of K rounds: positions/s measured directly")
+                         "re-rooting of both trees) instead of K rounds: positions/s measured directly; replaces --steps")
     ap.add_argument("--no-noise", action="store_true", help="searches without Dirichlet / Gumbel exploration noise")
     ap.add_argument("--eval-cache", type=int, default=0,
                     help="entries of the device-side evaluation cache (per-game scope; 0 = off, the default and the headline)")
@@ -457,7 +486,15 @@ def main():
                     help="size of the engine-wide child-slot page pool as a fraction of n_trees * slot_cap (1.0 = static worst case)")
     ap.add_argument("--no-extras", action="store_true",
                     help="skip the sub-records of the default run (the other BASELINE configurations at N=1, the real generation at N>1)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed region, write rank 0's root statistics (what gaz_root_dense hands a caller) as DIR/*.npy")
     args = ap.parse_args()
+    if args.moves > 0 and args.steps is not None:
+        ap.error("--moves M times M whole moves and replaces --steps; give one of them")
+    if args.steps is None:
+        args.steps = 40
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     cfg = dict(CONFIGS[args.config])
     if args.impl == "reference":
         return run_reference(args, cfg)
@@ -579,7 +616,8 @@ def measure(args, cfg, world, rank, local, peaks, want_cpu, full):
     import torch.distributed as dist
     n_games = args.games or cfg["games"]
 
-    sb = SelfPlayBench(cfg, n_games, local, noise=not args.no_noise, pool_fraction=args.pool_fraction, eval_cache=args.eval_cache)
+    sb = SelfPlayBench(cfg, n_games, local, noise=not args.no_noise, pool_fraction=args.pool_fraction, eval_cache=args.eval_cache,
+                       keep_roots=full and rank == 0 and bool(args.dump_outputs))
     sb.start()
     presearch = 0 if args.moves > 0 else args.presearch
     if presearch < 0:
@@ -629,6 +667,8 @@ def measure(args, cfg, world, rank, local, peaks, want_cpu, full):
 
     if args.moves > 0:
         line = run_moves(args, cfg, sb, timed_moves, barrier, world, rank, local, n_games)
+        if full and rank == 0 and args.dump_outputs:
+            dump_outputs(sb, args.dump_outputs)
         sb.eng.close()
         sb.net.close()
         del sb
@@ -655,6 +695,9 @@ def measure(args, cfg, world, rank, local, peaks, want_cpu, full):
     status = sb.eng.status()
     if status != 0:
         raise SystemExit("engine status %d (1 node overflow, 2 slot overflow, 4 LUT miss, 8 bad state)" % status)
+    if full and rank == 0 and args.dump_outputs:
+        dump_outputs(sb, args.dump_outputs)
+        sb.keep_roots = False     # the measurements below copy back only what they need
 
     # ---- one WHOLE move of every game, timed: fresh start position, the full run (forced root expansions included), root
     # statistics, the tau = 0 move, do_action / check_win, prune_tree of both trees, the next run's begin

@@ -1,8 +1,7 @@
 """Import the UNMODIFIED reference from /root/reference (TEST INFRASTRUCTURE ONLY).
 
 Works only in the build container (the GPU box has no /root/reference); used by
-oracle/gen_golden.py to produce tests/golden/*.json and by the optional
-reference-vs-oracle tests (skipped when the reference is absent).
+oracle/gen_golden.py, gen_cache_golden.py and gen_selfplay_golden.py to produce fixtures under tests/golden/.
 Recipe: SURVEY.md section 8(c).
 """
 import os

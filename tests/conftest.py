@@ -11,7 +11,6 @@ sys.path.insert(0, os.path.join(ROOT, "oracle"))
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run with -m gpu on the B200 box)")
-    config.addinivalue_line("markers", "reference: needs /root/reference (build container only)")
 
 
 def has_gpu():
