@@ -261,12 +261,26 @@ def finalize_games(game_obj, games, device=0, lib=None, tables=None, chunk_posit
 
 
 # ---------------------------------------------------------------------------------------- the batched driver --
+def match_tree_nets(game_ids):
+    """Network of each PUCT tree in a match, uint8 (len(game_ids), 2): tree k of the game with global id g searches with
+    network (k + g) % 2.  Tree 0 plays player -1, who moves first from the empty board, so network 0 moves first in the
+    even games and network 1 in the odd ones."""
+    g = np.asarray(game_ids, dtype=np.int64).reshape(-1, 1)
+    return ((g + np.arange(2)) % 2).astype(np.uint8)
+
+
 class BatchedSelfPlay:
-    """Plays the games `game_ids` (global ids) on one device, `n_slots` at a time."""
+    """Plays the games `game_ids` (global ids) on one device, `n_slots` at a time.
+
+    Matches (arena.play_match): `opponent = (spec_b, weights_b)` attaches a second network and every game's two PUCT trees
+    search with different networks (match_tree_nets); `openings(game_id) -> (board, next_player, action id history)`
+    seats that position instead of the empty board; `limits = (la, lb)` are the iteration limits of network 0's and
+    network 1's trees (default `self.limit` for both).  The finished records of a match also hold the played action ids
+    and the iterations of every search."""
 
     def __init__(self, game_class, build_config, train_config, game_ids, n_slots, device=0, evaluator="net",
                  spec=None, weights=None, seed=0, lib=None, hash_salt=0, node_cap=None, slot_cap=None,
-                 use_noise=True, slot_pool_fraction=None):
+                 use_noise=True, slot_pool_fraction=None, opponent=None, openings=None, limits=None):
         self.game_class = game_class
         self.proto = game_class()
         self.name = G.game_name_of(self.proto)
@@ -281,11 +295,20 @@ class BatchedSelfPlay:
         self.hash_salt = hash_salt
         limit = train_config["MCTS_iteration_limit"]
         self.limit = int(limit) if self.gumbel else int(limit * 1.5)          # Self_Play.py:99
+        self.match = opponent is not None
+        if self.match and self.gumbel:
+            raise ValueError("a match needs two PUCT trees per game (one per network); use_gumbel runs one tree per game")
+        if self.match and evaluator != "net":
+            raise ValueError("a match needs evaluator='net'")
+        self.openings = openings
+        self.limits = None if limits is None else (int(limits[0]), int(limits[1]))
+        self.tree_net = np.zeros((self.n_slots, self.tpg), np.uint8)   # network of every tree (all 0 outside a match)
+        search_limit = self.limit if self.limits is None else max(self.limits)
         self.max_actions = int(train_config["max_actions"])
         stablemax = bool(build_config.get("use_stablemax"))
         L = 7 if self.name == "connect4" else self.P
         # iterations a PUCT run can really make: `iteration_limit < n_legal -> 3 * n_legal` (MCTS.py:543-546)
-        self.eff_limit = self.limit if (self.gumbel or self.limit >= L) else 3 * L
+        self.eff_limit = search_limit if (self.gumbel or search_limit >= L) else 3 * L
         if node_cap is None:
             # Pools are sized for the tail of WHOLE games, not for the opening: an expansion whose position has terminal
             # replies creates a terminal parent and its k terminal children (MCTS.py:367-428), and the sub-tree kept
@@ -312,11 +335,15 @@ class BatchedSelfPlay:
         # are to the reference, Self_Play.py:233-235); "eval_cache_shared": one table for all games instead of per-game entries
         if int(train_config.get("eval_cache_entries", 0) or 0) > 0:
             self.eng.enable_eval_cache(int(train_config["eval_cache_entries"]), shared=bool(train_config.get("eval_cache_shared", False)))
-        self.net = None
+        self.net = self.net_b = None
         if evaluator == "net":
             from .net import Net
             self.net = Net(spec, weights, max_batch=self.n_slots, device=device)  # larger request lists are served in chunks
-            self.net.attach(self.eng)
+            if self.match:
+                self.net_b = Net(opponent[0], opponent[1], max_batch=self.n_slots, device=device)
+                self.eng.attach_nets([self.net, self.net_b])
+            else:
+                self.net.attach(self.eng)
         if not self.gumbel and use_noise:
             self.eng.set_noise(float(train_config.get("dirichlet_alpha", 0.3)), 0.25, seed)   # Self_Play.py:38-46
         self.use_gumbel_noise = self.gumbel and use_noise
@@ -355,11 +382,18 @@ class BatchedSelfPlay:
             gid = self.queue.pop(0)
             self.slot_game[s] = gid
             self.rngs[s] = np.random.Generator(np.random.PCG64([self.seed, int(gid)]))
-            self.traj[s] = dict(states=[], policies=[], q=[], z=[])
-            self.eng.set_game(int(s), np.zeros((self.H, self.W), np.int8), -1, [])
+            self.traj[s] = dict(states=[], policies=[], q=[], z=[], actions=[], iterations=[])
+            if self.openings is None:
+                self.eng.set_game(int(s), np.zeros((self.H, self.W), np.int8), -1, [])
+            else:
+                board, next_player, history = self.openings(int(gid))
+                self.eng.set_game(int(s), board, next_player, list(history))
             seated.append(s)
         keys = np.repeat(np.where(self.slot_game >= 0, self.slot_game, 0).astype(np.uint64), self.tpg)
         self.eng.set_tree_keys(keys * np.uint64(2) + np.tile(np.arange(self.tpg, dtype=np.uint64), self.n_slots))
+        if self.match:   # before the new roots below are evaluated
+            self.tree_net = match_tree_nets(np.where(self.slot_game >= 0, self.slot_game, 0))
+            self.eng.set_tree_nets(self.tree_net.reshape(-1))
         if seated:
             mask = np.zeros((self.n_slots, self.tpg), np.uint8)
             mask[seated] = 1
@@ -414,7 +448,9 @@ class BatchedSelfPlay:
         hist_len = ginfo[:, 1]
         run_tree = np.zeros(self.n_slots, np.int64) if self.gumbel else (mover > 0).astype(np.int64)
         limits = np.zeros((self.n_slots, self.tpg), np.int32)
-        limits[np.arange(self.n_slots), run_tree] = np.where(live, self.limit, 0)
+        run_limit = self.limit if self.limits is None else \
+            np.asarray(self.limits, np.int32)[self.tree_net[np.arange(self.n_slots), run_tree]]
+        limits[np.arange(self.n_slots), run_tree] = np.where(live, run_limit, 0)
         if self.use_gumbel_noise:   # MCTS_Gumbel.py:592-594: Gumbel(0,1) on the root logits, one stream per game
             noise = np.zeros((self.n_slots, 256), np.float64)
             for s in np.nonzero(live)[0]:
@@ -456,6 +492,7 @@ class BatchedSelfPlay:
             t["policies"].append(policy)
             t["q"].append(np.float32(q))
             t["z"].append(float(mover[s]))
+            t["iterations"].append(int(tinfo[s, 2]))
             if hist_len[s] == 0 and self.tc.get("opening_actions", False):               # Self_Play.py:130-140
                 acts, weights = zip(*self.tc["opening_actions"])
                 acts = [G.action_to_id(self.name, x) for x in acts]
@@ -465,12 +502,13 @@ class BatchedSelfPlay:
                     weights.append(1.0 - sum(weights))
                 a = int(acts[int(self.rngs[s].choice(len(acts), p=np.asarray(weights) / sum(weights)))])
             actions[s] = a
+            t["actions"].append(a)
         winners = e.apply_actions(actions)
         self.moves += int(live.sum())
         done = []
         for s in np.nonzero(live)[0]:
             w = int(winners[s])
-            n_act = len(self.traj[s]["z"])
+            n_act = int(hist_len[s]) + 1      # plies of the game, an opening seated by `openings` included
             if n_act >= self.max_actions:
                 w = 0      # Self_Play.py:155-157: `if actions_count == max_actions: winner = 0` - a WIN on that ply is a draw too
             if w != -2:
@@ -485,10 +523,13 @@ class BatchedSelfPlay:
             self._relieve_full_pools(cont, -mover)
         for s, w in done:
             t = self.traj[s]
-            self.finished.append(dict(game_id=int(self.slot_game[s]), winner=w, length=len(t["z"]),
-                                      states=np.asarray(t["states"], dtype=np.int8),
-                                      policies=np.asarray(t["policies"], dtype=np.float32),
-                                      q=np.asarray(t["q"], dtype=np.float32), z=np.asarray(t["z"], dtype=np.float32)))
+            rec = dict(game_id=int(self.slot_game[s]), winner=w, length=len(t["z"]),
+                       states=np.asarray(t["states"], dtype=np.int8),
+                       policies=np.asarray(t["policies"], dtype=np.float32),
+                       q=np.asarray(t["q"], dtype=np.float32), z=np.asarray(t["z"], dtype=np.float32))
+            if self.match:
+                rec.update(actions=np.asarray(t["actions"], dtype=np.int16), iterations=np.asarray(t["iterations"], dtype=np.int32))
+            self.finished.append(rec)
             self.traj[s] = None
         if done_slots:
             self._seat(done_slots)
@@ -506,8 +547,9 @@ class BatchedSelfPlay:
 
     def close(self):
         self.eng.close()
-        if self.net is not None:
-            self.net.close()
+        for n in (self.net, self.net_b):
+            if n is not None:
+                n.close()
 
 
 # ------------------------------------------------------------------------------------------- trajectory gather --

@@ -28,6 +28,8 @@ SYMBOLS = {
     "gaz_net_destroy": (None, [_P]),
     "gaz_net_forward_host": (C.c_int, [_P, _P, C.c_int, _P, _P, _P]),
     "gaz_attach_net": (C.c_int, [_P, _P]),
+    "gaz_attach_nets": (C.c_int, [_P, _P, C.c_int]),
+    "gaz_set_tree_nets": (C.c_int, [_P, _P]),
     "gaz_eval_net": (C.c_int, [_P]),
     "gaz_rounds_net": (C.c_int, [_P, C.c_int]),
     "gaz_rounds_net_async": (C.c_int, [_P, C.c_int]),

@@ -500,6 +500,7 @@ static int launch_hash(gaz_engine *e, uint64_t salt, int logits) {
     return 0;
 }
 int gaz_internal_launch_select(gaz_engine *e) { return launch_select(e); }
+int gaz_internal_alloc(gaz_engine *e, void **p, size_t bytes) { return ealloc(e, (uint8_t **)p, bytes); }
 int gaz_internal_launch_expand(gaz_engine *e) { return launch_expand(e); }
 static int read_leaf_count(gaz_engine *e) {
     int32_t n = 0;
@@ -530,10 +531,14 @@ int gaz_create(const gaz_config *cfg, gaz_engine **out) {
     gaz_engine *e = new gaz_engine();
     e->cfg = *cfg;
     e->bytes = 0;
-    e->net = nullptr;
+    e->nets[0] = e->nets[1] = nullptr;
+    e->n_nets = 0;
+    e->d_tree_net = nullptr;
+    e->route = nullptr;
     e->cache = nullptr;
     e->leaf_bound = 0;
-    e->round_graph = nullptr; e->round_graph_net = nullptr; e->round_graph_chunks = 0; e->round_graph_warm = 0;
+    e->round_graph = nullptr; e->round_graph_chunks = 0; e->round_graph_warm = 0;
+    e->attach_epoch = 0; e->round_graph_attach = 0;
     e->view_epoch = 0; e->round_graph_epoch = 0;
     View &v = e->v;
     memset(&v, 0, sizeof v);
@@ -626,6 +631,7 @@ void gaz_destroy(gaz_engine *e) {
 #endif
     for (void *p : e->allocs) dev_free(p);
     delete e->cache;
+    delete e->route;
 #ifndef GAZ_EMUL
     if (e->ev0) { cudaEventDestroy(e->ev0); cudaEventDestroy(e->ev1); }
     cudaStreamDestroy(e->stream);
@@ -1171,6 +1177,8 @@ int gaz_augment(int device, const int8_t *states, const float *policies, int64_t
 int gaz_eval_cache_enable(gaz_engine *e, int64_t entries, int shared_scope) {
     if (!e) return fail("null engine");
     if (e->cache) return fail("the evaluation cache is already enabled");
+    // the cache key does not include the network: a hit could hand one network's output to the other's trees
+    if (e->n_nets > 1) return fail("the evaluation cache cannot be used with two attached networks");
     if (entries < 1024) return fail("evaluation cache: at least 1024 entries");
     const View &v = e->v;
     gaz_eval_cache *c = new gaz_eval_cache();

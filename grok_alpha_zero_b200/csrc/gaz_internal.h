@@ -53,12 +53,17 @@ struct gaz_engine {
     gaz_stream_t stream;
     int64_t bytes;
     std::vector<void *> allocs;
-    struct gaz_net *net; // attached evaluator (gaz_net.cu) or null
+    // attached evaluators (gaz_net.cu): n_nets == 0 none, 1 every leaf goes to nets[0], 2 the leaves of tree t go to
+    // nets[tree_net[t]] (gaz_attach_nets / gaz_set_tree_nets)
+    struct gaz_net *nets[2];
+    int n_nets;
+    uint8_t *d_tree_net;   // [n_trees], allocated with the route buffers
+    struct gaz_route *route; // packed per-network leaf lists, or null until two networks were attached
     struct gaz_eval_cache *cache; // evaluation cache or null
     int leaf_bound;      // host-side upper bound of outstanding leaf requests (0 = n_trees)
     // CUDA graph of one search round (select -> network -> expand), built by gaz_net.cu on first use
     void *round_graph;   // cudaGraphExec_t
-    void *round_graph_net;
+    unsigned attach_epoch, round_graph_attach; // bumped by every attach: the graph bakes in the attached network set
     int round_graph_chunks, round_graph_warm;
     // Kernels take the View BY VALUE, so a captured graph bakes in the hyper-parameters and pointers of its capture time.
     // Every setter that changes e->v bumps view_epoch; run_rounds re-captures when the graph's epoch is stale.
@@ -108,6 +113,18 @@ struct gaz_eval_cache {
 // look-up pass over the current leaf list / fill pass after the evaluator served the packed misses (stream-ordered)
 int gaz_internal_cache_lookup(gaz_engine *e);
 int gaz_internal_cache_fill(gaz_engine *e);
+
+// Two attached networks (a match): every round the leaf list is partitioned by the network of each leaf's tree, each
+// network serves its own packed list and the outputs are scattered back to the leaf order (gaz_net.cu).
+struct gaz_route {
+    int32_t *idx[2];     // [n_trees]: leaf index of packed leaf m of network k
+    int32_t *count;      // [2] device counts
+    int8_t *state[2];    // [n_trees][S]
+    float *pol[2];       // [n_trees][P]
+    float *val[2];       // [n_trees]
+};
+// engine-owned device allocation (counted in gaz_bytes_allocated, freed with the engine)
+int gaz_internal_alloc(gaz_engine *e, void **p, size_t bytes);
 
 int gaz_internal_launch_select(gaz_engine *e);
 int gaz_internal_launch_expand(gaz_engine *e);

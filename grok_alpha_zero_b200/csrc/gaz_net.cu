@@ -366,6 +366,71 @@ __global__ void chunk_count_kernel(const int32_t *total, int offset, int max, in
     *out = c < 0 ? 0 : (c > max ? max : c);
 }
 
+// ---- two attached networks (gaz_attach_nets): route the leaf list by network, serve each packed list, scatter back
+// Stable partition of the round's leaf list by tree_net[tree of the leaf]: network k gets the ascending leaf indices of its
+// leaves in idx_k and their number in counts[k].  One CTA (a round has at most n_trees <= 32768 leaves) walks tiles of 1024
+// leaves, one per thread; the rank of a leaf among the network-1 leaves comes from a ballot + a scan of the 32 warp sums.
+__global__ void __launch_bounds__(1024) route_leaves_kernel(const gaz::LeafRec *leaves, const int32_t *leaf_count,
+                                                            const uint8_t *tree_net, int32_t *idx0, int32_t *idx1,
+                                                            int32_t *counts) {
+    __shared__ int warp_ones[32];
+    __shared__ int carry;   // network-1 leaves in the earlier tiles
+    const int n = *leaf_count, lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+    if (threadIdx.x == 0) carry = 0;
+    __syncthreads();
+    for (int base = 0; base < n; base += 1024) {
+        const int i = base + (int)threadIdx.x;
+        const bool one = i < n && tree_net[leaves[i].tree] != 0;
+        const unsigned b = __ballot_sync(0xffffffffu, one);
+        if (lane == 0) warp_ones[wid] = __popc(b);
+        __syncthreads();
+        int before = carry, tile = 0;
+        for (int w = 0; w < 32; w++) {
+            const int c = warp_ones[w];
+            before += w < wid ? c : 0;
+            tile += c;
+        }
+        before += __popc(b & ((1u << lane) - 1u));
+        if (i < n) {
+            if (one) idx1[before] = i;
+            else idx0[i - before] = i;
+        }
+        __syncthreads();
+        if (threadIdx.x == 0) carry += tile;
+        __syncthreads();
+    }
+    if (threadIdx.x == 0) { counts[0] = n - carry; counts[1] = carry; }
+}
+
+// warp per packed leaf (network 0's list, then network 1's): the input state of leaf idx_k[m] becomes packed row m of network k
+__global__ void __launch_bounds__(128) route_states_kernel(const int8_t *leaf_state, int S, const int32_t *counts,
+                                                           const int32_t *idx0, const int32_t *idx1, int8_t *st0, int8_t *st1) {
+    const int r = (int)((blockIdx.x * blockDim.x + threadIdx.x) >> 5), lane = threadIdx.x & 31;
+    const int c0 = counts[0];
+    if (r >= c0 + counts[1]) return;
+    const bool one = r >= c0;
+    const int m = one ? r - c0 : r;
+    const int8_t *src = leaf_state + (size_t)(one ? idx1 : idx0)[m] * S;
+    int8_t *dst = (one ? st1 : st0) + (size_t)m * S;
+    for (int j = lane; j < S; j += 32) dst[j] = src[j];
+}
+
+// warp per packed leaf: network k's policy row / value of packed leaf m go back to leaf idx_k[m] of the request list
+__global__ void __launch_bounds__(128) scatter_evals_kernel(int P, const int32_t *counts, const int32_t *idx0, const int32_t *idx1,
+                                                            const float *pol0, const float *pol1, const float *val0,
+                                                            const float *val1, float *policy, float *value) {
+    const int r = (int)((blockIdx.x * blockDim.x + threadIdx.x) >> 5), lane = threadIdx.x & 31;
+    const int c0 = counts[0];
+    if (r >= c0 + counts[1]) return;
+    const bool one = r >= c0;
+    const int m = one ? r - c0 : r;
+    const int leaf = (one ? idx1 : idx0)[m];
+    const float *src = (one ? pol1 : pol0) + (size_t)m * P;
+    float *dst = policy + (size_t)leaf * P;
+    for (int j = lane; j < P; j += 32) dst[j] = src[j];
+    if (lane == 0) value[leaf] = (one ? val1 : val0)[m];
+}
+
 // ====================================================================== executor ==
 typedef CUresult (*PFN_encodeTiled)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *,
                                     const cuuint64_t *, const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave,
@@ -1411,43 +1476,113 @@ int gaz_net_forward_host(gaz_net *n, const int8_t *states, int cnt, float *polic
     return cnt;
 }
 
+static void drop_round_graph(gaz_engine *e) {
+    if (e->round_graph) { cudaGraphExecDestroy((cudaGraphExec_t)e->round_graph); e->round_graph = nullptr; }
+    e->round_graph_warm = 0;
+    e->attach_epoch++;
+}
+
 int gaz_attach_net(gaz_engine *e, gaz_net *n) {
     if (!e) return gaz_fail("null engine");
     if (n) {
         if (n->game != e->cfg.game) return gaz_fail("network game %d != engine game %d", n->game, e->cfg.game);
     }
-    e->net = n;
-    if (e->round_graph) { cudaGraphExecDestroy((cudaGraphExec_t)e->round_graph); e->round_graph = nullptr; }
-    e->round_graph_warm = 0;
+    e->nets[0] = n;
+    e->nets[1] = nullptr;
+    e->n_nets = n ? 1 : 0;
+    drop_round_graph(e);
+    return 0;
+}
+
+int gaz_attach_nets(gaz_engine *e, gaz_net *const *nets, int n_nets) {
+    if (!e || !nets) return gaz_fail("null argument");
+    if (n_nets == 1) return gaz_attach_net(e, nets[0]);
+    if (n_nets != 2) return gaz_fail("gaz_attach_nets: %d networks (1 or 2)", n_nets);
+    if (!nets[0] || !nets[1]) return gaz_fail("gaz_attach_nets: null network");
+    if (nets[0]->game != nets[1]->game) return gaz_fail("the two networks are for different games (%d, %d)", nets[0]->game, nets[1]->game);
+    if (nets[0]->game != e->cfg.game) return gaz_fail("network game %d != engine game %d", nets[0]->game, e->cfg.game);
+    if (nets[0]->P != nets[1]->P || nets[0]->P != e->v.P)
+        return gaz_fail("the two networks have policy sizes %d and %d (engine %d)", nets[0]->P, nets[1]->P, e->v.P);
+    if (e->cache) return gaz_fail("two networks cannot share the evaluation cache: its key does not include the network");
+    if (!e->route) {
+        const size_t NT = (size_t)e->v.n_trees, S = (size_t)e->v.ncell * e->v.C, P = (size_t)e->v.P;
+        gaz_route r;
+        int rc = 0;
+        for (int k = 0; k < 2; k++) {
+            rc |= gaz_internal_alloc(e, (void **)&r.idx[k], NT * sizeof(int32_t));
+            rc |= gaz_internal_alloc(e, (void **)&r.state[k], NT * S);
+            rc |= gaz_internal_alloc(e, (void **)&r.pol[k], NT * P * sizeof(float));
+            rc |= gaz_internal_alloc(e, (void **)&r.val[k], NT * sizeof(float));
+        }
+        rc |= gaz_internal_alloc(e, (void **)&r.count, 2 * sizeof(int32_t));
+        rc |= gaz_internal_alloc(e, (void **)&e->d_tree_net, NT);   // zero: every tree on network 0
+        if (rc != 0) return -1;
+        e->route = new gaz_route(r);
+    }
+    e->nets[0] = nets[0];
+    e->nets[1] = nets[1];
+    e->n_nets = 2;
+    drop_round_graph(e);
+    return 0;
+}
+
+int gaz_set_tree_nets(gaz_engine *e, const uint8_t *tree_net) {
+    if (!e || !tree_net) return gaz_fail("null argument");
+    const int lim = e->n_nets > 1 ? e->n_nets : 1;
+    for (int t = 0; t < e->v.n_trees; t++)
+        if (tree_net[t] >= lim) return gaz_fail("tree_net[%d] = %d, but %d network(s) attached", t, (int)tree_net[t], e->n_nets);
+    if (!e->d_tree_net) return 0;   // no second network was ever attached: every tree is on network 0 already
+    CKN(cudaMemcpyAsync(e->d_tree_net, tree_net, (size_t)e->v.n_trees, cudaMemcpyHostToDevice, e->stream));
+    return 0;
+}
+
+// forward chunks of network n over a packed request list of at most leaf_bound leaves (the count itself is on the device)
+static int forward_chunks(gaz_engine *e, gaz_net *n, const int32_t *total, const int8_t *states, float *pol, float *val) {
+    const gaz::View &v = e->v;
+    const int bound = e->leaf_bound > 0 ? e->leaf_bound : v.n_trees;
+    const int chunks = (bound + n->max_batch - 1) / n->max_batch;
+    if (chunks > 16) return gaz_fail("leaf bound %d needs more than 16 chunks of %d", bound, n->max_batch);
+    const size_t ss = (size_t)v.ncell * v.C;
+    for (int ck = 0; ck < chunks; ck++) {
+        const int off = ck * n->max_batch;
+        chunk_count_kernel<<<1, 1, 0, e->stream>>>(total, off, n->max_batch, n->d_chunk_count + ck);
+        if (net_forward(n, states + (size_t)off * ss, n->d_chunk_count + ck, pol + (size_t)off * v.P, val + off, e->stream) != 0) return -1;
+    }
     return 0;
 }
 
 // Serves the engine's outstanding leaf requests; the request list is cut into chunks of max_batch
 // leaves (the host-side bound e->leaf_bound says how many chunks can be non-empty).
 static int engine_forward(gaz_engine *e) {
-    gaz_net *n = e->net;
     const gaz::View &v = e->v;
-    int bound = e->leaf_bound > 0 ? e->leaf_bound : v.n_trees;
-    int chunks = (bound + n->max_batch - 1) / n->max_batch;
-    if (chunks > 16) return gaz_fail("leaf bound %d needs more than 16 chunks of %d", bound, n->max_batch);
-    const size_t ss = (size_t)v.ncell * v.C;
+    if (e->n_nets == 2) {
+        // route -> network 0's chunks -> network 1's chunks -> scatter.  Either packed list can hold every leaf, so each
+        // network gets the chunks of the whole bound and a changed tree_net needs no new round graph.
+        gaz_route *r = e->route;
+        const unsigned rows = (unsigned)(((size_t)v.n_trees * 32 + 127) / 128);
+        route_leaves_kernel<<<1, 1024, 0, e->stream>>>(v.leaves, v.leaf_count, e->d_tree_net, r->idx[0], r->idx[1], r->count);
+        route_states_kernel<<<rows, 128, 0, e->stream>>>(v.leaf_state, v.ncell * v.C, r->count, r->idx[0], r->idx[1], r->state[0], r->state[1]);
+        CKN(cudaGetLastError());
+        for (int k = 0; k < 2; k++)
+            if (forward_chunks(e, e->nets[k], r->count + k, r->state[k], r->pol[k], r->val[k]) != 0) return -1;
+        scatter_evals_kernel<<<rows, 128, 0, e->stream>>>(v.P, r->count, r->idx[0], r->idx[1], r->pol[0], r->pol[1], r->val[0],
+                                                          r->val[1], v.policy, v.value);
+        CKN(cudaGetLastError());
+        return 0;
+    }
     // with the evaluation cache on, the network sees the packed misses of the look-up pass instead of the leaf list
     gaz_eval_cache *c = e->cache;
     if (c && gaz_internal_cache_lookup(e) != 0) return -1;
     const int32_t *total = c ? c->miss_count : v.leaf_count;
     const int8_t *states = c ? c->packed_state : v.leaf_state;
     float *pol = c ? c->packed_pol : v.policy, *val = c ? c->packed_val : v.value;
-    for (int ck = 0; ck < chunks; ck++) {
-        const int off = ck * n->max_batch;
-        chunk_count_kernel<<<1, 1, 0, e->stream>>>(total, off, n->max_batch, n->d_chunk_count + ck);
-        if (net_forward(n, states + (size_t)off * ss, n->d_chunk_count + ck, pol + (size_t)off * v.P, val + off, e->stream) != 0) return -1;
-    }
+    if (forward_chunks(e, e->nets[0], total, states, pol, val) != 0) return -1;
     if (c && gaz_internal_cache_fill(e) != 0) return -1;
     return 0;
 }
 
 int gaz_eval_net(gaz_engine *e) {
-    if (!e || !e->net) return gaz_fail("no network attached");
+    if (!e || !e->n_nets) return gaz_fail("no network attached");
     return engine_forward(e);
 }
 
@@ -1460,15 +1595,19 @@ static int one_round_eager(gaz_engine *e) {
 // n_rounds x (select -> network -> expand).  One round is ~30-45 kernel launches; for small networks (TicTacToe: 0.2 ms of
 // GPU work per round) the launch path is the bottleneck, so the round is captured once into a CUDA graph and replayed.
 // Every kernel reads its leaf count from device memory, so the graph does not depend on the data; it is rebuilt when
-// the number of forward chunks or the attached network changes.  Disabled while conv launches are being event-timed.
+// the number of forward chunks or the attached network set changes.  Disabled while conv launches are being event-timed.
 static int run_rounds(gaz_engine *e, int n_rounds) {
-    gaz_net *n = e->net;
-    const bool use_graph = !n->profile;   // per-launch event timers need eager launches
+    bool profiling = false;
+    int chunks = 0;   // forward chunks of every attached network, 8 bits each
+    const int bound = e->leaf_bound > 0 ? e->leaf_bound : e->v.n_trees;
+    for (int k = 0; k < e->n_nets; k++) {
+        profiling = profiling || e->nets[k]->profile;
+        chunks |= ((bound + e->nets[k]->max_batch - 1) / e->nets[k]->max_batch) << (8 * k);
+    }
+    const bool use_graph = !profiling;   // per-launch event timers need eager launches
     for (int r = 0; r < n_rounds; r++) {
         if (!use_graph) { if (one_round_eager(e) != 0) return -1; continue; }
-        const int bound = e->leaf_bound > 0 ? e->leaf_bound : e->v.n_trees;
-        const int chunks = (bound + n->max_batch - 1) / n->max_batch;
-        if (!e->round_graph || e->round_graph_chunks != chunks || e->round_graph_net != (void *)n ||
+        if (!e->round_graph || e->round_graph_chunks != chunks || e->round_graph_attach != e->attach_epoch ||
             e->round_graph_epoch != e->view_epoch) {
             if (e->round_graph_warm < 1) { // first round eagerly: one-time function attributes are set outside a capture
                 if (one_round_eager(e) != 0) return -1;
@@ -1487,7 +1626,7 @@ static int run_rounds(gaz_engine *e, int n_rounds) {
             if (ce != cudaSuccess) return gaz_fail("cudaGraphInstantiate: %s", cudaGetErrorString(ce));
             e->round_graph = (void *)ex;
             e->round_graph_chunks = chunks;
-            e->round_graph_net = (void *)n;
+            e->round_graph_attach = e->attach_epoch;
             e->round_graph_epoch = e->view_epoch;
         }
         CKN(cudaGraphLaunch((cudaGraphExec_t)e->round_graph, e->stream));
@@ -1496,7 +1635,7 @@ static int run_rounds(gaz_engine *e, int n_rounds) {
 }
 
 int gaz_rounds_net(gaz_engine *e, int n_rounds) {
-    if (!e || !e->net) return gaz_fail("no network attached");
+    if (!e || !e->n_nets) return gaz_fail("no network attached");
     if (run_rounds(e, n_rounds) != 0) return -1;
     CKN(cudaStreamSynchronize(e->stream));
     return 0;
@@ -1504,7 +1643,7 @@ int gaz_rounds_net(gaz_engine *e, int n_rounds) {
 
 // same without the trailing synchronise (bench: events bracket many calls)
 int gaz_rounds_net_async(gaz_engine *e, int n_rounds) {
-    if (!e || !e->net) return gaz_fail("no network attached");
+    if (!e || !e->n_nets) return gaz_fail("no network attached");
     return run_rounds(e, n_rounds);
 }
 

@@ -228,6 +228,19 @@ class Engine:
     def eval_net(self):
         self._ck(self.lib.gaz_eval_net(self._h))
 
+    def attach_nets(self, nets):
+        """Attach one or two `net.Net` evaluators of this game.  With two, the leaves of tree t are served by
+        nets[tree_net[t]] (set_tree_nets; every tree starts on network 0); the evaluation cache cannot be on."""
+        nets = list(nets)
+        hs = (C.c_void_p * len(nets))(*[n._h.value for n in nets])
+        self._ck(self.lib.gaz_attach_nets(self._h, hs, len(nets)))
+        self._net = nets  # keep alive
+
+    def set_tree_nets(self, tree_net):
+        """network index (< number of attached networks) of every tree, uint8 (n_trees,)"""
+        t = np.ascontiguousarray(np.broadcast_to(np.asarray(tree_net), (self.n_trees,)), dtype=np.uint8)
+        self._ck(self.lib.gaz_set_tree_nets(self._h, _p(t)))
+
     def rounds_net(self, n, sync=True):
         fn = self.lib.gaz_rounds_net if sync else self.lib.gaz_rounds_net_async
         self._ck(fn(self._h, int(n)))

@@ -68,6 +68,13 @@ int gaz_net_forward_host(gaz_net *net, const int8_t *states, int n, float *polic
 /* Attach to an engine: gaz_eval_net() then serves the outstanding leaf requests of gaz_select()
  * on the engine's stream with no host round trip. */
 int gaz_attach_net(gaz_engine *e, gaz_net *net);
+/* Self_Play.py:39-57 keeps one tree per player; for a match each tree's leaves go to the network of its side.
+ * nets: n_nets (1 or 2) networks of the engine's game.  n_nets == 1 is gaz_attach_net(e, nets[0]).  Two networks must
+ * have the same policy size and cannot be combined with the evaluation cache (its key does not include the network). */
+int gaz_attach_nets(gaz_engine *e, gaz_net *const *nets, int n_nets);
+/* tree_net: n_trees bytes, network index of every tree (< n_nets).  Stream-ordered upload; a captured round graph stays
+ * valid (it reads the table from device memory). */
+int gaz_set_tree_nets(gaz_engine *e, const uint8_t *tree_net);
 int gaz_eval_net(gaz_engine *e);
 /* n_rounds x (select -> network -> expand), stream-ordered, no host sync inside; returns 0 */
 int gaz_rounds_net(gaz_engine *e, int n_rounds);
