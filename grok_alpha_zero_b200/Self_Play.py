@@ -272,15 +272,18 @@ def match_tree_nets(game_ids):
 class BatchedSelfPlay:
     """Plays the games `game_ids` (global ids) on one device, `n_slots` at a time.
 
-    Matches (arena.play_match): `opponent = (spec_b, weights_b)` attaches a second network and every game's two PUCT trees
-    search with different networks (match_tree_nets); `openings(game_id) -> (board, next_player, action id history)`
-    seats that position instead of the empty board; `limits = (la, lb)` are the iteration limits of network 0's and
-    network 1's trees (default `self.limit` for both).  The finished records of a match also hold the played action ids
-    and the iterations of every search."""
+    Matches and tournaments (arena.play_match / arena.play_tournament): `opponents = [(spec_k, weights_k), ...]` attaches
+    networks 1..K-1 (K <= 8; network 0 is `spec` / `weights`), and `tree_nets(game_id) -> (network of tree 0, network of
+    tree 1)` says which network each of a game's two PUCT trees searches with.  `opponent = (spec_b, weights_b)` is
+    `opponents = [opponent]` with `tree_nets` = match_tree_nets.  Networks of equal specs share one activation workspace
+    (net.Net(share=...)).  `openings(game_id) -> (board, next_player, action id history)` seats that position instead of
+    the empty board; `limits` are the K per-network iteration limits (default `self.limit` for every network).  The finished
+    records of a match also hold the played action ids and the iterations of every search."""
 
     def __init__(self, game_class, build_config, train_config, game_ids, n_slots, device=0, evaluator="net",
                  spec=None, weights=None, seed=0, lib=None, hash_salt=0, node_cap=None, slot_cap=None,
-                 use_noise=True, slot_pool_fraction=None, opponent=None, openings=None, limits=None):
+                 use_noise=True, slot_pool_fraction=None, opponent=None, openings=None, limits=None, opponents=None,
+                 tree_nets=None):
         self.game_class = game_class
         self.proto = game_class()
         self.name = G.game_name_of(self.proto)
@@ -295,13 +298,26 @@ class BatchedSelfPlay:
         self.hash_salt = hash_salt
         limit = train_config["MCTS_iteration_limit"]
         self.limit = int(limit) if self.gumbel else int(limit * 1.5)          # Self_Play.py:99
-        self.match = opponent is not None
+        if opponent is not None:
+            if opponents is not None:
+                raise ValueError("pass either opponent or opponents")
+            opponents, tree_nets = [opponent], None
+        self.opponents = [] if opponents is None else list(opponents)
+        self.n_nets = 1 + len(self.opponents)
+        self.match = self.n_nets > 1
+        if self.n_nets > 8:
+            raise ValueError("at most 8 networks, got %d" % self.n_nets)
         if self.match and self.gumbel:
             raise ValueError("a match needs two PUCT trees per game (one per network); use_gumbel runs one tree per game")
         if self.match and evaluator != "net":
             raise ValueError("a match needs evaluator='net'")
+        if tree_nets is None and self.n_nets > 2:
+            raise ValueError("%d networks need tree_nets(game_id)" % self.n_nets)
+        self.tree_nets_of = tree_nets          # None: match_tree_nets
         self.openings = openings
-        self.limits = None if limits is None else (int(limits[0]), int(limits[1]))
+        if limits is not None and len(limits) != self.n_nets:
+            raise ValueError("limits: %d values for %d networks" % (len(limits), self.n_nets))
+        self.limits = None if limits is None else tuple(int(x) for x in limits)
         self.tree_net = np.zeros((self.n_slots, self.tpg), np.uint8)   # network of every tree (all 0 outside a match)
         search_limit = self.limit if self.limits is None else max(self.limits)
         self.max_actions = int(train_config["max_actions"])
@@ -335,15 +351,18 @@ class BatchedSelfPlay:
         # are to the reference, Self_Play.py:233-235); "eval_cache_shared": one table for all games instead of per-game entries
         if int(train_config.get("eval_cache_entries", 0) or 0) > 0:
             self.eng.enable_eval_cache(int(train_config["eval_cache_entries"]), shared=bool(train_config.get("eval_cache_shared", False)))
-        self.net = self.net_b = None
+        self.nets = []
         if evaluator == "net":
             from .net import Net
-            self.net = Net(spec, weights, max_batch=self.n_slots, device=device)  # larger request lists are served in chunks
+            for sp_k, w_k in [(spec, weights)] + self.opponents:
+                donor = next((n for n in self.nets if n.spec == sp_k), None)    # attached networks run one after another
+                # larger request lists are served in chunks
+                self.nets.append(Net(sp_k, w_k, max_batch=self.n_slots, device=device, share=donor))
             if self.match:
-                self.net_b = Net(opponent[0], opponent[1], max_batch=self.n_slots, device=device)
-                self.eng.attach_nets([self.net, self.net_b])
+                self.eng.attach_nets(self.nets)
             else:
-                self.net.attach(self.eng)
+                self.nets[0].attach(self.eng)
+        self.net = self.nets[0] if self.nets else None
         if not self.gumbel and use_noise:
             self.eng.set_noise(float(train_config.get("dirichlet_alpha", 0.3)), 0.25, seed)   # Self_Play.py:38-46
         self.use_gumbel_noise = self.gumbel and use_noise
@@ -392,7 +411,11 @@ class BatchedSelfPlay:
         keys = np.repeat(np.where(self.slot_game >= 0, self.slot_game, 0).astype(np.uint64), self.tpg)
         self.eng.set_tree_keys(keys * np.uint64(2) + np.tile(np.arange(self.tpg, dtype=np.uint64), self.n_slots))
         if self.match:   # before the new roots below are evaluated
-            self.tree_net = match_tree_nets(np.where(self.slot_game >= 0, self.slot_game, 0))
+            if self.tree_nets_of is None:
+                self.tree_net = match_tree_nets(np.where(self.slot_game >= 0, self.slot_game, 0))
+            else:        # idle slots search nothing; their trees stay on network 0
+                self.tree_net = np.array([self.tree_nets_of(int(g)) if g >= 0 else (0, 0) for g in self.slot_game],
+                                         np.uint8).reshape(self.n_slots, 2)
             self.eng.set_tree_nets(self.tree_net.reshape(-1))
         if seated:
             mask = np.zeros((self.n_slots, self.tpg), np.uint8)
@@ -547,9 +570,8 @@ class BatchedSelfPlay:
 
     def close(self):
         self.eng.close()
-        for n in (self.net, self.net_b):
-            if n is not None:
-                n.close()
+        for n in self.nets:
+            n.close()
 
 
 # ------------------------------------------------------------------------------------------- trajectory gather --

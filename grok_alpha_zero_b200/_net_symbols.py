@@ -25,6 +25,7 @@ class GazNetDesc(C.Structure):
 
 SYMBOLS = {
     "gaz_net_create": (C.c_int, [C.POINTER(GazNetDesc), C.POINTER(_P)]),
+    "gaz_net_create_shared": (C.c_int, [C.POINTER(GazNetDesc), _P, C.POINTER(_P)]),
     "gaz_net_destroy": (None, [_P]),
     "gaz_net_forward_host": (C.c_int, [_P, _P, C.c_int, _P, _P, _P]),
     "gaz_attach_net": (C.c_int, [_P, _P]),

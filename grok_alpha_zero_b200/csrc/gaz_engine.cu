@@ -512,7 +512,7 @@ static int read_leaf_count(gaz_engine *e) {
 extern "C" {
 
 const char *gaz_last_error(void) { return g_err.c_str(); }
-int gaz_abi_version(void) { return 2; }
+int gaz_abi_version(void) { return 3; }
 
 int gaz_create(const gaz_config *cfg, gaz_engine **out) {
     if (!cfg || !out) return fail("null argument");
@@ -531,8 +531,9 @@ int gaz_create(const gaz_config *cfg, gaz_engine **out) {
     gaz_engine *e = new gaz_engine();
     e->cfg = *cfg;
     e->bytes = 0;
-    e->nets[0] = e->nets[1] = nullptr;
+    for (int k = 0; k < GAZ_MAX_NETS; k++) e->nets[k] = nullptr;
     e->n_nets = 0;
+    e->tree_net_max = 0;
     e->d_tree_net = nullptr;
     e->route = nullptr;
     e->cache = nullptr;
@@ -1178,7 +1179,7 @@ int gaz_eval_cache_enable(gaz_engine *e, int64_t entries, int shared_scope) {
     if (!e) return fail("null engine");
     if (e->cache) return fail("the evaluation cache is already enabled");
     // the cache key does not include the network: a hit could hand one network's output to the other's trees
-    if (e->n_nets > 1) return fail("the evaluation cache cannot be used with two attached networks");
+    if (e->n_nets > 1) return fail("the evaluation cache cannot be used with more than one attached network");
     if (entries < 1024) return fail("evaluation cache: at least 1024 entries");
     const View &v = e->v;
     gaz_eval_cache *c = new gaz_eval_cache();

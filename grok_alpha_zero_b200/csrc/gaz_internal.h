@@ -1,6 +1,7 @@
 // gaz_internal.h -- engine internals shared by gaz_engine.cu and gaz_net.cu (not part of the ABI).
 #pragma once
 #include "../../include/gaz_b200.h"
+#include "../../include/gaz_net.h"
 #include "gaz_core.cuh"
 
 #include <string>
@@ -53,18 +54,20 @@ struct gaz_engine {
     gaz_stream_t stream;
     int64_t bytes;
     std::vector<void *> allocs;
-    // attached evaluators (gaz_net.cu): n_nets == 0 none, 1 every leaf goes to nets[0], 2 the leaves of tree t go to
+    // attached evaluators (gaz_net.cu): n_nets == 0 none, 1 every leaf goes to nets[0], >= 2 the leaves of tree t go to
     // nets[tree_net[t]] (gaz_attach_nets / gaz_set_tree_nets)
-    struct gaz_net *nets[2];
+    struct gaz_net *nets[GAZ_MAX_NETS];
     int n_nets;
     uint8_t *d_tree_net;   // [n_trees], allocated with the route buffers
+    int tree_net_max;      // largest index in the uploaded table (host copy)
     struct gaz_route *route; // packed per-network leaf lists, or null until two networks were attached
     struct gaz_eval_cache *cache; // evaluation cache or null
     int leaf_bound;      // host-side upper bound of outstanding leaf requests (0 = n_trees)
     // CUDA graph of one search round (select -> network -> expand), built by gaz_net.cu on first use
     void *round_graph;   // cudaGraphExec_t
     unsigned attach_epoch, round_graph_attach; // bumped by every attach: the graph bakes in the attached network set
-    int round_graph_chunks, round_graph_warm;
+    uint64_t round_graph_chunks; // forward chunks of every attached network, 8 bits per network
+    int round_graph_warm;
     // Kernels take the View BY VALUE, so a captured graph bakes in the hyper-parameters and pointers of its capture time.
     // Every setter that changes e->v bumps view_epoch; run_rounds re-captures when the graph's epoch is stale.
     unsigned view_epoch, round_graph_epoch;
@@ -114,14 +117,16 @@ struct gaz_eval_cache {
 int gaz_internal_cache_lookup(gaz_engine *e);
 int gaz_internal_cache_fill(gaz_engine *e);
 
-// Two attached networks (a match): every round the leaf list is partitioned by the network of each leaf's tree, each
-// network serves its own packed list and the outputs are scattered back to the leaf order (gaz_net.cu).
+// Several attached networks (a match, a tournament): every round the leaf list is partitioned by the network of each
+// leaf's tree, each network serves its own packed list and the outputs are scattered back to the leaf order (gaz_net.cu).
+// Lists 0..n_alloc-1 are allocated; attaching more networks later allocates the missing ones.
 struct gaz_route {
-    int32_t *idx[2];     // [n_trees]: leaf index of packed leaf m of network k
-    int32_t *count;      // [2] device counts
-    int8_t *state[2];    // [n_trees][S]
-    float *pol[2];       // [n_trees][P]
-    float *val[2];       // [n_trees]
+    int n_alloc;
+    int32_t *idx[GAZ_MAX_NETS];   // [n_trees]: leaf index of packed leaf m of network k
+    int32_t *count;               // [GAZ_MAX_NETS] device counts
+    int8_t *state[GAZ_MAX_NETS];  // [n_trees][S]
+    float *pol[GAZ_MAX_NETS];     // [n_trees][P]
+    float *val[GAZ_MAX_NETS];     // [n_trees]
 };
 // engine-owned device allocation (counted in gaz_bytes_allocated, freed with the engine)
 int gaz_internal_alloc(gaz_engine *e, void **p, size_t bytes);

@@ -366,69 +366,78 @@ __global__ void chunk_count_kernel(const int32_t *total, int offset, int max, in
     *out = c < 0 ? 0 : (c > max ? max : c);
 }
 
-// ---- two attached networks (gaz_attach_nets): route the leaf list by network, serve each packed list, scatter back
-// Stable partition of the round's leaf list by tree_net[tree of the leaf]: network k gets the ascending leaf indices of its
-// leaves in idx_k and their number in counts[k].  One CTA (a round has at most n_trees <= 32768 leaves) walks tiles of 1024
-// leaves, one per thread; the rank of a leaf among the network-1 leaves comes from a ballot + a scan of the 32 warp sums.
+// ---- several attached networks (gaz_attach_nets): route the leaf list by network, serve each packed list, scatter back
+// Stable K-way partition of the round's leaf list by tree_net[tree of the leaf]: network k gets the ascending leaf indices of
+// its leaves in r.idx[k] and their number in r.count[k].  One CTA (a round has at most n_trees <= 32768 leaves) walks tiles
+// of 1024 leaves, one per thread.  In a tile, a leaf's rank among the same-network leaves of its warp comes from
+// __match_any_sync; the per-warp per-network counts are scanned (warp k scans network k's 32 warp counts) and added to the
+// network's carry from the earlier tiles.
 __global__ void __launch_bounds__(1024) route_leaves_kernel(const gaz::LeafRec *leaves, const int32_t *leaf_count,
-                                                            const uint8_t *tree_net, int32_t *idx0, int32_t *idx1,
-                                                            int32_t *counts) {
-    __shared__ int warp_ones[32];
-    __shared__ int carry;   // network-1 leaves in the earlier tiles
+                                                            const uint8_t *tree_net, int K, const gaz_route r) {
+    __shared__ int off[GAZ_MAX_NETS][32];   // leaves of network k in warp w of the tile, then their first packed index
+    __shared__ int carry[GAZ_MAX_NETS];     // leaves of network k in the earlier tiles
+    __shared__ int tile[GAZ_MAX_NETS];
     const int n = *leaf_count, lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-    if (threadIdx.x == 0) carry = 0;
-    __syncthreads();
+    if (threadIdx.x < GAZ_MAX_NETS) carry[threadIdx.x] = 0;
     for (int base = 0; base < n; base += 1024) {
+        if (threadIdx.x < GAZ_MAX_NETS * 32) off[threadIdx.x >> 5][threadIdx.x & 31] = 0;
+        __syncthreads();
         const int i = base + (int)threadIdx.x;
-        const bool one = i < n && tree_net[leaves[i].tree] != 0;
-        const unsigned b = __ballot_sync(0xffffffffu, one);
-        if (lane == 0) warp_ones[wid] = __popc(b);
+        const int k = i < n ? (int)tree_net[leaves[i].tree] : GAZ_MAX_NETS;   // lanes past the end form a group of their own
+        const unsigned peers = __match_any_sync(0xffffffffu, k);
+        const int rank = __popc(peers & ((1u << lane) - 1u));
+        if (k < K && rank == 0) off[k][wid] = __popc(peers);
         __syncthreads();
-        int before = carry, tile = 0;
-        for (int w = 0; w < 32; w++) {
-            const int c = warp_ones[w];
-            before += w < wid ? c : 0;
-            tile += c;
-        }
-        before += __popc(b & ((1u << lane) - 1u));
-        if (i < n) {
-            if (one) idx1[before] = i;
-            else idx0[i - before] = i;
+        if (wid < K) {
+            const int c = off[wid][lane];
+            int x = c;
+            for (int d = 1; d < 32; d <<= 1) {
+                const int y = __shfl_up_sync(0xffffffffu, x, d);
+                if (lane >= d) x += y;
+            }
+            off[wid][lane] = carry[wid] + x - c;
+            if (lane == 31) tile[wid] = x;
         }
         __syncthreads();
-        if (threadIdx.x == 0) carry += tile;
+        if (k < K) r.idx[k][off[k][wid] + rank] = i;
+        if (threadIdx.x < K) carry[threadIdx.x] += tile[threadIdx.x];
         __syncthreads();
     }
-    if (threadIdx.x == 0) { counts[0] = n - carry; counts[1] = carry; }
+    __syncthreads();
+    if (threadIdx.x < K) r.count[threadIdx.x] = carry[threadIdx.x];
 }
 
-// warp per packed leaf (network 0's list, then network 1's): the input state of leaf idx_k[m] becomes packed row m of network k
-__global__ void __launch_bounds__(128) route_states_kernel(const int8_t *leaf_state, int S, const int32_t *counts,
-                                                           const int32_t *idx0, const int32_t *idx1, int8_t *st0, int8_t *st1) {
-    const int r = (int)((blockIdx.x * blockDim.x + threadIdx.x) >> 5), lane = threadIdx.x & 31;
-    const int c0 = counts[0];
-    if (r >= c0 + counts[1]) return;
-    const bool one = r >= c0;
-    const int m = one ? r - c0 : r;
-    const int8_t *src = leaf_state + (size_t)(one ? idx1 : idx0)[m] * S;
-    int8_t *dst = (one ? st1 : st0) + (size_t)m * S;
+// packed row `row` of the concatenated lists (network 0's, then network 1's, ...) -> its network k and index m in k's list
+__device__ __forceinline__ bool route_row(const int32_t *count, int K, int row, int &k, int &m) {
+    int base = 0;
+    for (k = 0; k < K; k++) {
+        const int c = count[k];
+        if (row < base + c) { m = row - base; return true; }
+        base += c;
+    }
+    return false;
+}
+
+// warp per packed leaf: the input state of leaf idx_k[m] becomes packed row m of network k
+__global__ void __launch_bounds__(128) route_states_kernel(const int8_t *leaf_state, int S, int K, const gaz_route r) {
+    const int row = (int)((blockIdx.x * blockDim.x + threadIdx.x) >> 5), lane = threadIdx.x & 31;
+    int k, m;
+    if (!route_row(r.count, K, row, k, m)) return;
+    const int8_t *src = leaf_state + (size_t)r.idx[k][m] * S;
+    int8_t *dst = r.state[k] + (size_t)m * S;
     for (int j = lane; j < S; j += 32) dst[j] = src[j];
 }
 
 // warp per packed leaf: network k's policy row / value of packed leaf m go back to leaf idx_k[m] of the request list
-__global__ void __launch_bounds__(128) scatter_evals_kernel(int P, const int32_t *counts, const int32_t *idx0, const int32_t *idx1,
-                                                            const float *pol0, const float *pol1, const float *val0,
-                                                            const float *val1, float *policy, float *value) {
-    const int r = (int)((blockIdx.x * blockDim.x + threadIdx.x) >> 5), lane = threadIdx.x & 31;
-    const int c0 = counts[0];
-    if (r >= c0 + counts[1]) return;
-    const bool one = r >= c0;
-    const int m = one ? r - c0 : r;
-    const int leaf = (one ? idx1 : idx0)[m];
-    const float *src = (one ? pol1 : pol0) + (size_t)m * P;
+__global__ void __launch_bounds__(128) scatter_evals_kernel(int P, int K, const gaz_route r, float *policy, float *value) {
+    const int row = (int)((blockIdx.x * blockDim.x + threadIdx.x) >> 5), lane = threadIdx.x & 31;
+    int k, m;
+    if (!route_row(r.count, K, row, k, m)) return;
+    const int leaf = r.idx[k][m];
+    const float *src = r.pol[k] + (size_t)m * P;
     float *dst = policy + (size_t)leaf * P;
     for (int j = lane; j < P; j += 32) dst[j] = src[j];
-    if (lane == 0) value[leaf] = (one ? val1 : val0)[m];
+    if (lane == 0) value[leaf] = r.val[k][m];
 }
 
 // ====================================================================== executor ==
@@ -480,8 +489,18 @@ struct NetOp {
     long long rows_dense;
 };
 
+// Activation workspace: every allocation of a network that scales with max_batch, in creation order.  Networks of one
+// structure make the same allocations in the same order, so gaz_net_create_shared hands the i-th of them to the sharer.
+// Reference-counted; freed with the last network that uses it.
+struct NetWorkspace {
+    int refs;
+    std::vector<void *> ptrs;
+    std::vector<size_t> bytes;
+};
+
 struct gaz_net {
     int game, H, W, Cin, P, Wp, P_pad, max_batch, policy_mode, device;
+    NetWorkspace *ws;
     long long rows_alloc;
     std::vector<NetBuf> bufs;
     std::vector<NetOp> ops;
@@ -494,7 +513,7 @@ struct gaz_net {
     cudaEvent_t ev_fork, ev_join;
     gaz_block::TrunkArgs *trunk_args;   // host staging of a trunk launch's arguments
     int head1_begin, head2_begin;  // op indices: first op of the first / second head; head2_begin = 0: the heads are not separable
-    // own I/O buffers for the host path
+    // I/O buffers for the host path (workspace)
     int8_t *d_states;
     int32_t *d_count;
     int32_t *d_chunk_count; // [16] per-chunk leaf counts of an engine-driven forward
@@ -877,8 +896,33 @@ static int net_forward(gaz_net *n, const int8_t *states, const int32_t *count, f
 
 extern "C" {
 
-int gaz_net_create(const gaz_net_desc *desc, gaz_net **out) {
+// first structural difference between `desc` and network `s`, or 0 if a network of `desc` may share s's workspace
+static int structure_mismatch(const gaz_net_desc *desc, const gaz_net *s) {
+    if (desc->game != s->game) return gaz_fail("shared workspace: game %d != %d", desc->game, s->game);
+    if (desc->device != s->device) return gaz_fail("shared workspace: device %d != %d", desc->device, s->device);
+    if (desc->max_batch != s->max_batch) return gaz_fail("shared workspace: max_batch %d != %d", desc->max_batch, s->max_batch);
+    if (desc->n_bufs != (int)s->bufs.size()) return gaz_fail("shared workspace: %d buffers != %d", desc->n_bufs, (int)s->bufs.size());
+    for (int i = 0; i < desc->n_bufs; i++)
+        if (desc->bufs[i].kind != s->bufs[(size_t)i].kind || desc->bufs[i].width != s->bufs[(size_t)i].width)
+            return gaz_fail("shared workspace: buffer %d is (kind %d, width %d), the shared network's is (kind %d, width %d)", i,
+                            desc->bufs[i].kind, desc->bufs[i].width, s->bufs[(size_t)i].kind, s->bufs[(size_t)i].width);
+    if (desc->n_ops != (int)s->ops.size()) return gaz_fail("shared workspace: %d ops != %d", desc->n_ops, (int)s->ops.size());
+    for (int i = 0; i < desc->n_ops; i++) {
+        const gaz_net_op &a = desc->ops[i], &b = s->ops[(size_t)i].d;
+        const char *field = a.type != b.type ? "type" : a.in_buf != b.in_buf ? "in_buf" : a.res_buf != b.res_buf ? "res_buf"
+                          : a.out_raw != b.out_raw ? "out_raw" : a.out_a != b.out_a ? "out_a" : a.out_b != b.out_b ? "out_b"
+                          : a.cin != b.cin ? "cin" : a.cout != b.cout ? "cout" : a.ksize != b.ksize ? "ksize"
+                          : a.act != b.act ? "act" : a.flags != b.flags ? "flags" : nullptr;
+        if (field) return gaz_fail("shared workspace: op %d differs in %s from the shared network's", i, field);
+    }
+    return 0;
+}
+
+int gaz_net_create(const gaz_net_desc *desc, gaz_net **out) { return gaz_net_create_shared(desc, nullptr, out); }
+
+int gaz_net_create_shared(const gaz_net_desc *desc, gaz_net *share, gaz_net **out) {
     if (!desc || !out) return gaz_fail("null argument");
+    if (share && structure_mismatch(desc, share) != 0) return -1;
     int ndev = 0;
     cudaError_t ce = cudaGetDeviceCount(&ndev);
     if (ce != cudaSuccess || ndev <= 0) return gaz_fail("no CUDA device (%s): the network has no CPU path", cudaGetErrorString(ce));
@@ -892,6 +936,8 @@ int gaz_net_create(const gaz_net_desc *desc, gaz_net **out) {
         enc = (PFN_encodeTiled)fn;
     }
     gaz_net *n = new gaz_net();
+    if (share) { n->ws = share->ws; n->ws->refs++; }
+    else { n->ws = new NetWorkspace(); n->ws->refs = 1; }
     n->game = desc->game;
     if (desc->game == GAZ_GAME_TICTACTOE) { n->H = 3; n->W = 3; n->Cin = 2; n->P = 9; }
     else if (desc->game == GAZ_GAME_CONNECT4) { n->H = 6; n->W = 7; n->Cin = 4; n->P = 7; }
@@ -929,6 +975,19 @@ int gaz_net_create(const gaz_net_desc *desc, gaz_net **out) {
         n->bytes += (int64_t)bytes;
         return 0;
     };
+    size_t ws_next = 0;   // allocations of the workspace taken so far
+    auto walloc = [&](void **p, size_t bytes) -> int {
+        if (share) {
+            if (ws_next >= n->ws->ptrs.size() || n->ws->bytes[ws_next] != bytes)
+                return gaz_fail("shared workspace: activation allocation %d (%zu bytes) has no match", (int)ws_next, bytes);
+            *p = n->ws->ptrs[ws_next++];
+            return 0;
+        }
+        if (alloc(p, bytes) != 0) return -1;
+        n->ws->ptrs.push_back(*p);
+        n->ws->bytes.push_back(bytes);
+        return 0;
+    };
     int rc = 0;
     rc |= alloc((void **)&n->wf, (size_t)desc->n_wf * 4);
     rc |= alloc((void **)&n->wh, (size_t)desc->n_wh * 2);
@@ -942,14 +1001,14 @@ int gaz_net_create(const gaz_net_desc *desc, gaz_net **out) {
         else if (b.kind == GAZ_BUF_ROWS_F32) b.bytes = (size_t)n->rows_alloc * b.width * 4;
         else b.bytes = (size_t)n->max_batch * b.width * 4;
         b.ptr = nullptr;
-        rc |= alloc(&b.ptr, b.bytes);
+        rc |= walloc(&b.ptr, b.bytes);
         n->bufs.push_back(b);
     }
-    rc |= alloc((void **)&n->d_states, (size_t)n->max_batch * n->H * n->W * n->Cin);
+    rc |= walloc((void **)&n->d_states, (size_t)n->max_batch * n->H * n->W * n->Cin);
     rc |= alloc((void **)&n->d_count, 16);
     rc |= alloc((void **)&n->d_chunk_count, 16 * 4);
-    rc |= alloc((void **)&n->d_policy, (size_t)n->max_batch * n->P * 4);
-    rc |= alloc((void **)&n->d_value, (size_t)n->max_batch * 4);
+    rc |= walloc((void **)&n->d_policy, (size_t)n->max_batch * n->P * 4);
+    rc |= walloc((void **)&n->d_value, (size_t)n->max_batch * 4);
     if (rc != 0) { gaz_net_destroy(n); return -1; }
     for (int i = 0; i < desc->n_ops; i++) {
         NetOp op;
@@ -1036,7 +1095,7 @@ int gaz_net_create(const gaz_net_desc *desc, gaz_net **out) {
         const int in_pad = (d.cin + 7) & ~7; // TMA row pitch must be a multiple of 16 bytes
         if (!((pr.d.cout == 8 && pr.d.ksize == 3) || (pr.d.cout == 4 && pr.d.ksize == 1))) continue; // headconv_board_kernel shapes
         op.rows_dense = (((long long)n->max_batch + 255) / 256) * 256;
-        if (alloc((void **)&op.d_act, (size_t)op.rows_dense * in_pad * 2) != 0) { gaz_net_destroy(n); return -1; }
+        if (walloc((void **)&op.d_act, (size_t)op.rows_dense * in_pad * 2) != 0) { gaz_net_destroy(n); return -1; }
         std::vector<uint16_t> wt((size_t)d.cout * in_pad, (uint16_t)0);
         for (int i = 0; i < d.cin; i++)
             for (int o = 0; o < d.cout; o++) {
@@ -1190,7 +1249,7 @@ int gaz_net_create(const gaz_net_desc *desc, gaz_net **out) {
             if (o.out_raw == d1.in_buf && o.out_a < 0 && !c2.d_xbf) src = &c2;
         }
         if (!src) continue;
-        if (alloc((void **)&src->d_xbf, (size_t)n->rows_alloc * 128 * 2) != 0) { gaz_net_destroy(n); return -1; }
+        if (walloc((void **)&src->d_xbf, (size_t)n->rows_alloc * 128 * 2) != 0) { gaz_net_destroy(n); return -1; }
         const size_t ld = (size_t)3 * d1.cin;
         std::vector<uint16_t> wt((size_t)48 * ld, 0);
         auto bf16_bits = [](float f) -> uint16_t { uint32_t u; memcpy(&u, &f, 4); return (uint16_t)((u + 0x7FFFu + ((u >> 16) & 1u)) >> 16); };
@@ -1440,6 +1499,10 @@ int gaz_net_create(const gaz_net_desc *desc, gaz_net **out) {
         if (ok) { n->head1_begin = h1; n->head2_begin = h2; }
     }
 #endif
+    if (share && ws_next != n->ws->ptrs.size()) {
+        gaz_net_destroy(n);
+        return gaz_fail("shared workspace: %d of its %d activation allocations used", (int)ws_next, (int)share->ws->ptrs.size());
+    }
     CKN(cudaDeviceSynchronize());
     *out = n;
     return 0;
@@ -1449,9 +1512,13 @@ void gaz_net_destroy(gaz_net *n) {
     if (!n) return;
     cudaStreamSynchronize(n->stream);
     cudaStreamSynchronize(n->stream2);
-    for (auto &b : n->bufs) cudaFree(b.ptr);
-    for (auto &op : n->ops) { if (op.d_se_b1) cudaFree(op.d_se_b1); if (op.d_act) cudaFree(op.d_act); if (op.d_wt) cudaFree(op.d_wt); if (op.d_stem_w) cudaFree(op.d_stem_w); if (op.d_stem_par) cudaFree(op.d_stem_par); if (op.d_frag) cudaFree(op.d_frag); if (op.d_hbias) cudaFree(op.d_hbias); if (op.d_xbf) cudaFree(op.d_xbf); if (op.d_frag0) cudaFree(op.d_frag0); }
-    cudaFree(n->wf); cudaFree(n->wh); cudaFree(n->d_states); cudaFree(n->d_count); cudaFree(n->d_chunk_count); cudaFree(n->d_policy); cudaFree(n->d_value);
+    // bufs, d_act, d_xbf and the host-path staging belong to the workspace
+    for (auto &op : n->ops) { if (op.d_se_b1) cudaFree(op.d_se_b1); if (op.d_wt) cudaFree(op.d_wt); if (op.d_stem_w) cudaFree(op.d_stem_w); if (op.d_stem_par) cudaFree(op.d_stem_par); if (op.d_frag) cudaFree(op.d_frag); if (op.d_hbias) cudaFree(op.d_hbias); if (op.d_frag0) cudaFree(op.d_frag0); }
+    cudaFree(n->wf); cudaFree(n->wh); cudaFree(n->d_count); cudaFree(n->d_chunk_count);
+    if (n->ws && --n->ws->refs == 0) {
+        for (void *p : n->ws->ptrs) cudaFree(p);
+        delete n->ws;
+    }
     for (auto e : n->ev) cudaEventDestroy(e);
     cudaStreamDestroy(n->stream);
     cudaStreamDestroy(n->stream2);
@@ -1487,8 +1554,7 @@ int gaz_attach_net(gaz_engine *e, gaz_net *n) {
     if (n) {
         if (n->game != e->cfg.game) return gaz_fail("network game %d != engine game %d", n->game, e->cfg.game);
     }
-    e->nets[0] = n;
-    e->nets[1] = nullptr;
+    for (int k = 0; k < GAZ_MAX_NETS; k++) e->nets[k] = k == 0 ? n : nullptr;
     e->n_nets = n ? 1 : 0;
     drop_round_graph(e);
     return 0;
@@ -1496,32 +1562,42 @@ int gaz_attach_net(gaz_engine *e, gaz_net *n) {
 
 int gaz_attach_nets(gaz_engine *e, gaz_net *const *nets, int n_nets) {
     if (!e || !nets) return gaz_fail("null argument");
+    if (n_nets < 1 || n_nets > GAZ_MAX_NETS) return gaz_fail("gaz_attach_nets: %d networks (1 to %d)", n_nets, GAZ_MAX_NETS);
+    for (int k = 0; k < n_nets; k++)
+        if (!nets[k]) return gaz_fail("gaz_attach_nets: network %d is null", k);
     if (n_nets == 1) return gaz_attach_net(e, nets[0]);
-    if (n_nets != 2) return gaz_fail("gaz_attach_nets: %d networks (1 or 2)", n_nets);
-    if (!nets[0] || !nets[1]) return gaz_fail("gaz_attach_nets: null network");
-    if (nets[0]->game != nets[1]->game) return gaz_fail("the two networks are for different games (%d, %d)", nets[0]->game, nets[1]->game);
+    for (int k = 1; k < n_nets; k++)
+        if (nets[k]->game != nets[0]->game)
+            return gaz_fail("networks 0 and %d are for different games (%d, %d)", k, nets[0]->game, nets[k]->game);
     if (nets[0]->game != e->cfg.game) return gaz_fail("network game %d != engine game %d", nets[0]->game, e->cfg.game);
-    if (nets[0]->P != nets[1]->P || nets[0]->P != e->v.P)
-        return gaz_fail("the two networks have policy sizes %d and %d (engine %d)", nets[0]->P, nets[1]->P, e->v.P);
-    if (e->cache) return gaz_fail("two networks cannot share the evaluation cache: its key does not include the network");
+    for (int k = 0; k < n_nets; k++)
+        if (nets[k]->P != e->v.P)
+            return gaz_fail("network %d has policy size %d (network 0: %d, engine: %d)", k, nets[k]->P, nets[0]->P, e->v.P);
+    if (e->cache) return gaz_fail("%d networks cannot share the evaluation cache: its key does not include the network", n_nets);
+    const size_t NT = (size_t)e->v.n_trees, S = (size_t)e->v.ncell * e->v.C, P = (size_t)e->v.P;
     if (!e->route) {
-        const size_t NT = (size_t)e->v.n_trees, S = (size_t)e->v.ncell * e->v.C, P = (size_t)e->v.P;
         gaz_route r;
-        int rc = 0;
-        for (int k = 0; k < 2; k++) {
-            rc |= gaz_internal_alloc(e, (void **)&r.idx[k], NT * sizeof(int32_t));
-            rc |= gaz_internal_alloc(e, (void **)&r.state[k], NT * S);
-            rc |= gaz_internal_alloc(e, (void **)&r.pol[k], NT * P * sizeof(float));
-            rc |= gaz_internal_alloc(e, (void **)&r.val[k], NT * sizeof(float));
-        }
-        rc |= gaz_internal_alloc(e, (void **)&r.count, 2 * sizeof(int32_t));
-        rc |= gaz_internal_alloc(e, (void **)&e->d_tree_net, NT);   // zero: every tree on network 0
-        if (rc != 0) return -1;
+        memset(&r, 0, sizeof r);
+        if (gaz_internal_alloc(e, (void **)&r.count, GAZ_MAX_NETS * sizeof(int32_t)) != 0 ||
+            gaz_internal_alloc(e, (void **)&e->d_tree_net, NT) != 0)   // zero: every tree on network 0
+            return -1;
         e->route = new gaz_route(r);
     }
-    e->nets[0] = nets[0];
-    e->nets[1] = nets[1];
-    e->n_nets = 2;
+    for (int k = e->route->n_alloc; k < n_nets; k++) {   // packed lists of the networks not seen before
+        gaz_route &r = *e->route;
+        if (gaz_internal_alloc(e, (void **)&r.idx[k], NT * sizeof(int32_t)) != 0 ||
+            gaz_internal_alloc(e, (void **)&r.state[k], NT * S) != 0 ||
+            gaz_internal_alloc(e, (void **)&r.pol[k], NT * P * sizeof(float)) != 0 ||
+            gaz_internal_alloc(e, (void **)&r.val[k], NT * sizeof(float)) != 0)
+            return -1;
+        r.n_alloc = k + 1;
+    }
+    if (e->tree_net_max >= n_nets) {   // the table names a network that is no longer attached: back to network 0
+        CKN(cudaMemsetAsync(e->d_tree_net, 0, NT, e->stream));
+        e->tree_net_max = 0;
+    }
+    for (int k = 0; k < GAZ_MAX_NETS; k++) e->nets[k] = k < n_nets ? nets[k] : nullptr;
+    e->n_nets = n_nets;
     drop_round_graph(e);
     return 0;
 }
@@ -1529,10 +1605,14 @@ int gaz_attach_nets(gaz_engine *e, gaz_net *const *nets, int n_nets) {
 int gaz_set_tree_nets(gaz_engine *e, const uint8_t *tree_net) {
     if (!e || !tree_net) return gaz_fail("null argument");
     const int lim = e->n_nets > 1 ? e->n_nets : 1;
-    for (int t = 0; t < e->v.n_trees; t++)
+    int mx = 0;
+    for (int t = 0; t < e->v.n_trees; t++) {
         if (tree_net[t] >= lim) return gaz_fail("tree_net[%d] = %d, but %d network(s) attached", t, (int)tree_net[t], e->n_nets);
+        mx = tree_net[t] > mx ? tree_net[t] : mx;
+    }
     if (!e->d_tree_net) return 0;   // no second network was ever attached: every tree is on network 0 already
     CKN(cudaMemcpyAsync(e->d_tree_net, tree_net, (size_t)e->v.n_trees, cudaMemcpyHostToDevice, e->stream));
+    e->tree_net_max = mx;
     return 0;
 }
 
@@ -1555,18 +1635,18 @@ static int forward_chunks(gaz_engine *e, gaz_net *n, const int32_t *total, const
 // leaves (the host-side bound e->leaf_bound says how many chunks can be non-empty).
 static int engine_forward(gaz_engine *e) {
     const gaz::View &v = e->v;
-    if (e->n_nets == 2) {
-        // route -> network 0's chunks -> network 1's chunks -> scatter.  Either packed list can hold every leaf, so each
-        // network gets the chunks of the whole bound and a changed tree_net needs no new round graph.
-        gaz_route *r = e->route;
+    if (e->n_nets > 1) {
+        // route -> each network's chunks in turn -> scatter.  Any packed list can hold every leaf, so each network gets the
+        // chunks of the whole bound and a changed tree_net needs no new round graph.
+        const gaz_route &r = *e->route;
+        const int K = e->n_nets;
         const unsigned rows = (unsigned)(((size_t)v.n_trees * 32 + 127) / 128);
-        route_leaves_kernel<<<1, 1024, 0, e->stream>>>(v.leaves, v.leaf_count, e->d_tree_net, r->idx[0], r->idx[1], r->count);
-        route_states_kernel<<<rows, 128, 0, e->stream>>>(v.leaf_state, v.ncell * v.C, r->count, r->idx[0], r->idx[1], r->state[0], r->state[1]);
+        route_leaves_kernel<<<1, 1024, 0, e->stream>>>(v.leaves, v.leaf_count, e->d_tree_net, K, r);
+        route_states_kernel<<<rows, 128, 0, e->stream>>>(v.leaf_state, v.ncell * v.C, K, r);
         CKN(cudaGetLastError());
-        for (int k = 0; k < 2; k++)
-            if (forward_chunks(e, e->nets[k], r->count + k, r->state[k], r->pol[k], r->val[k]) != 0) return -1;
-        scatter_evals_kernel<<<rows, 128, 0, e->stream>>>(v.P, r->count, r->idx[0], r->idx[1], r->pol[0], r->pol[1], r->val[0],
-                                                          r->val[1], v.policy, v.value);
+        for (int k = 0; k < K; k++)
+            if (forward_chunks(e, e->nets[k], r.count + k, r.state[k], r.pol[k], r.val[k]) != 0) return -1;
+        scatter_evals_kernel<<<rows, 128, 0, e->stream>>>(v.P, K, r, v.policy, v.value);
         CKN(cudaGetLastError());
         return 0;
     }
@@ -1598,11 +1678,11 @@ static int one_round_eager(gaz_engine *e) {
 // the number of forward chunks or the attached network set changes.  Disabled while conv launches are being event-timed.
 static int run_rounds(gaz_engine *e, int n_rounds) {
     bool profiling = false;
-    int chunks = 0;   // forward chunks of every attached network, 8 bits each
+    uint64_t chunks = 0;   // forward chunks of every attached network, 8 bits each (at most 16 chunks, 8 networks)
     const int bound = e->leaf_bound > 0 ? e->leaf_bound : e->v.n_trees;
     for (int k = 0; k < e->n_nets; k++) {
         profiling = profiling || e->nets[k]->profile;
-        chunks |= ((bound + e->nets[k]->max_batch - 1) / e->nets[k]->max_batch) << (8 * k);
+        chunks |= (uint64_t)((bound + e->nets[k]->max_batch - 1) / e->nets[k]->max_batch) << (8 * k);
     }
     const bool use_graph = !profiling;   // per-launch event timers need eager launches
     for (int r = 0; r < n_rounds; r++) {

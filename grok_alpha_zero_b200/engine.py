@@ -229,7 +229,7 @@ class Engine:
         self._ck(self.lib.gaz_eval_net(self._h))
 
     def attach_nets(self, nets):
-        """Attach one or two `net.Net` evaluators of this game.  With two, the leaves of tree t are served by
+        """Attach 1 to 8 `net.Net` evaluators of this game.  With several, the leaves of tree t are served by
         nets[tree_net[t]] (set_tree_nets; every tree starts on network 0); the evaluation cache cannot be on."""
         nets = list(nets)
         hs = (C.c_void_p * len(nets))(*[n._h.value for n in nets])

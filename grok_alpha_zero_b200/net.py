@@ -235,9 +235,14 @@ def check_weights(spec, W):
 
 class Net:
     """CUDA policy/value network.  `forward` is the host-buffer path (parity tests, mailbox server);
-    `attach(engine)` wires it to a search engine so leaves never leave HBM."""
+    `attach(engine)` wires it to a search engine so leaves never leave HBM.
 
-    def __init__(self, spec, weights, max_batch, device=0, lib=None):
+    `share=net` uses `net`'s activation workspace (everything that scales with `max_batch`) instead of allocating one: the
+    spec must be structurally the same (same game, layers and widths; the weights may differ), with the same `max_batch`
+    and device.  The workspace lives until the last network using it is closed.  Networks sharing a workspace must not run
+    forward passes at the same time; networks attached to one engine never do, and `forward` returns synchronised."""
+
+    def __init__(self, spec, weights, max_batch, device=0, lib=None, share=None):
         self.lib = lib if lib is not None else _lib.load()
         self.spec = spec
         self.H, self.W, self.Cin, self.P = spec["H"], spec["W"], spec["Cin"], spec["P"]
@@ -282,7 +287,9 @@ class Net:
                           wh.size)
         h = C.c_void_p()
         self._h = None
-        rc = self.lib.gaz_net_create(C.byref(desc), C.byref(h))
+        if share is not None and share._h is None:
+            raise ValueError("share: that network is closed")
+        rc = self.lib.gaz_net_create_shared(C.byref(desc), share._h if share is not None else None, C.byref(h))
         if rc < 0:
             raise EngineError(self.lib.gaz_last_error().decode())
         self._h = h

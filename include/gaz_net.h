@@ -22,6 +22,9 @@ extern "C" {
 
 typedef struct gaz_net gaz_net;
 
+/* most networks one engine can hold (gaz_attach_nets) */
+#define GAZ_MAX_NETS 8
+
 enum { GAZ_OP_STEM = 0, GAZ_OP_CONV_TC = 1, GAZ_OP_SE = 2, GAZ_OP_HEADCONV = 3, GAZ_OP_DENSE = 4, GAZ_OP_POLICY_OUT = 5 };
 enum { GAZ_BUF_ROWS_BF16 = 0, GAZ_BUF_ROWS_F32 = 1, GAZ_BUF_FLAT_F32 = 2 };
 enum { GAZ_ACT_NONE = 0, GAZ_ACT_RELU = 1, GAZ_ACT_GELU = 2, GAZ_ACT_TANH = 3 };
@@ -58,6 +61,16 @@ typedef struct gaz_net_desc {
 } gaz_net_desc;
 
 int gaz_net_create(const gaz_net_desc *desc, gaz_net **out);
+/* gaz_net_create, but the new network uses the activation workspace of `share` (share == NULL: gaz_net_create): every
+ * allocation that scales with max_batch (the activation buffers, the bf16 trunk copy of a tensor-core head, the dense
+ * layers' bf16 inputs and the host-forward staging).  Weights, per-op tables, streams, events and the per-chunk counters
+ * stay the network's own.  `share` must have the same game, device and max_batch, the same buffer list (kind, width) and
+ * the same op structure (type, buffer ids, cin, cout, ksize, act, flags); otherwise the call fails naming the first
+ * difference.  The workspace is reference-counted: it lives until the last network using it is destroyed, in any order.
+ * Rule: networks that share a workspace must not run forward passes at the same time.  Networks attached to one engine
+ * serve a round one after another on the engine's stream, and gaz_net_forward_host synchronises before it returns, so
+ * both uses are safe from one host thread. */
+int gaz_net_create_shared(const gaz_net_desc *desc, gaz_net *share, gaz_net **out);
 void gaz_net_destroy(gaz_net *net);
 
 /* session.run(["policy","value"], {"inputs": x}) for a host batch (MCTS.py:224-235,
@@ -68,9 +81,12 @@ int gaz_net_forward_host(gaz_net *net, const int8_t *states, int n, float *polic
 /* Attach to an engine: gaz_eval_net() then serves the outstanding leaf requests of gaz_select()
  * on the engine's stream with no host round trip. */
 int gaz_attach_net(gaz_engine *e, gaz_net *net);
-/* Self_Play.py:39-57 keeps one tree per player; for a match each tree's leaves go to the network of its side.
- * nets: n_nets (1 or 2) networks of the engine's game.  n_nets == 1 is gaz_attach_net(e, nets[0]).  Two networks must
- * have the same policy size and cannot be combined with the evaluation cache (its key does not include the network). */
+/* Self_Play.py:39-57 keeps one tree per player; in a match or a tournament each tree's leaves go to the network of its
+ * side.  nets: n_nets (1..GAZ_MAX_NETS) non-null networks of the engine's game.  n_nets == 1 is gaz_attach_net(e, nets[0]).
+ * Several networks must have the same policy size and cannot be combined with the evaluation cache (its key does not
+ * include the network).  Every round, the leaf list is partitioned by network (stable), each network serves its packed
+ * list in chunks of the whole leaf bound, and the outputs are scattered back to leaf order.  A refused call changes
+ * nothing.  Attaching fewer networks than the tree table names resets the table to network 0. */
 int gaz_attach_nets(gaz_engine *e, gaz_net *const *nets, int n_nets);
 /* tree_net: n_trees bytes, network index of every tree (< n_nets).  Stream-ordered upload; a captured round graph stays
  * valid (it reads the table from device memory). */
@@ -86,6 +102,7 @@ int gaz_rounds_net_async(gaz_engine *e, int n_rounds);
  * pairs to keep; 0 disables) and read the totals back after a stream synchronise. */
 int gaz_net_profile(gaz_net *net, int max_launches);
 int gaz_net_profile_read(gaz_net *net, float *total_ms, int *n_launches, float *per_op_ms);
+/* device bytes the network allocated itself (a shared activation workspace counts for its creator only) */
 int64_t gaz_net_bytes(gaz_net *net);
 int gaz_net_launches_per_forward(gaz_net *net);
 /* residual blocks run by the launch of op `op`: consecutive fused blocks share one launch of up to 6 layers (gaz_block.cuh);

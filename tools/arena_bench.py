@@ -54,10 +54,10 @@ def timed(args, spec, wa, wb):
 
 
 def routing_time(sp):
-    """one more match move with eager rounds (Net.profile switches graph replay off) under torch.profiler"""
+    """one more move with eager rounds (Net.profile switches graph replay off) under torch.profiler"""
     import torch
     from torch.profiler import ProfilerActivity, profile
-    for n in (sp.net, sp.net_b):
+    for n in sp.nets:
         n.profile(1)
     torch.cuda.init()
     with profile(activities=[ProfilerActivity.CUDA, ProfilerActivity.CPU]) as prof:
