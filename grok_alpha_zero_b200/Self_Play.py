@@ -278,7 +278,9 @@ class BatchedSelfPlay:
     `opponents = [opponent]` with `tree_nets` = match_tree_nets.  Networks of equal specs share one activation workspace
     (net.Net(share=...)).  `openings(game_id) -> (board, next_player, action id history)` seats that position instead of
     the empty board; `limits` are the K per-network iteration limits (default `self.limit` for every network).  The finished
-    records of a match also hold the played action ids and the iterations of every search."""
+    records of a match also hold the played action ids and the iterations of every search.  `train_config["eval_symmetry"]`
+    ("none" by default: the reference's evaluation; "random" or "ensemble", seeded from `seed`) is how every network evaluates
+    (Engine.set_eval_symmetry)."""
 
     def __init__(self, game_class, build_config, train_config, game_ids, n_slots, device=0, evaluator="net",
                  spec=None, weights=None, seed=0, lib=None, hash_salt=0, node_cap=None, slot_cap=None,
@@ -363,6 +365,14 @@ class BatchedSelfPlay:
             else:
                 self.nets[0].attach(self.eng)
         self.net = self.nets[0] if self.nets else None
+        # train_config["eval_symmetry"]: "none" (default, the reference's evaluation), "random" (each request under one board
+        # symmetry drawn from a hash of the seed, the game's global id and the position) or "ensemble" (the mean over all
+        # symmetries, n times the network work); only "none" keeps reference parity (Engine.set_eval_symmetry)
+        sym = str(train_config.get("eval_symmetry", "none") or "none")
+        if sym != "none":
+            if evaluator != "net":
+                raise ValueError("eval_symmetry=%r needs evaluator='net'" % sym)
+            self.eng.set_eval_symmetry(sym, seed)
         if not self.gumbel and use_noise:
             self.eng.set_noise(float(train_config.get("dirichlet_alpha", 0.3)), 0.25, seed)   # Self_Play.py:38-46
         self.use_gumbel_noise = self.gumbel and use_noise
@@ -666,7 +676,8 @@ def run_self_play(game_class, configs, folder_path, per_process_wait_time=1e-3, 
     """Same call as the reference's `run_self_play(game_class, configs, folder_path, per_process_wait_time)`; plays
     `games_per_generation - game_stats[2]` games (resume rule of Self_Play.py:267-272) on this rank's share of the
     game ids and appends them to `folder_path/Self_Play_Data` on rank 0.  Extra keys read from train_config:
-    `games_per_gpu` (concurrent games per GPU, default 4096).  `weights`: Keras-layout dict or a checkpoint path
+    `games_per_gpu` (concurrent games per GPU, default 4096) and `eval_symmetry` ("none", the default and the reference's
+    evaluation; "random" or "ensemble", see BatchedSelfPlay - seeded from `seed`, and not reference parity).  `weights`: Keras-layout dict or a checkpoint path
     (default `folder_path/model.npz`, else random init).  `seed`: None draws one from the OS on rank 0 (the reference
     reseeds every worker from entropy, Self_Play.py:221) and broadcasts it; an explicit seed makes a run reproducible.
     `evaluator`: "net" (CUDA network), "hash" (deterministic parity evaluator) or "random" - a uniform-random policy /

@@ -31,6 +31,7 @@ SYMBOLS = {
     "gaz_attach_net": (C.c_int, [_P, _P]),
     "gaz_attach_nets": (C.c_int, [_P, _P, C.c_int]),
     "gaz_set_tree_nets": (C.c_int, [_P, _P]),
+    "gaz_set_eval_symmetry": (C.c_int, [_P, C.c_int, C.c_int, _P, _P, C.c_uint64]),
     "gaz_eval_net": (C.c_int, [_P]),
     "gaz_rounds_net": (C.c_int, [_P, C.c_int]),
     "gaz_rounds_net_async": (C.c_int, [_P, C.c_int]),

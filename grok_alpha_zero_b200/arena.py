@@ -77,11 +77,11 @@ def opening_book(game_class, plies, seed):
     return opening
 
 
-def _match_config(game_class, configs, n_nets, iterations, opening_plies):
+def _match_config(game_class, configs, n_nets, iterations, opening_plies, symmetry):
     """(game name, build config, train config of the match, exploration on?, per-network iteration limits, opening plies)"""
     build_config, train_config = configs[0], configs[1]
     name = G.game_name_of(game_class())
-    tc = dict(train_config)
+    tc = dict(train_config, eval_symmetry=symmetry)
     explore = bool(tc.get("match_exploration", False))
     if not explore:
         tc.update(num_explore_actions_first=0, num_explore_actions_second=0, opening_actions=False)
@@ -114,7 +114,7 @@ def tally(outcomes, colour_keys=("a_first", "a_second")):
 
 
 def play_match(game_class, configs, weights_a, weights_b, n_games, spec_b=None, iterations=None, opening_plies=None, seed=0,
-               device=0, n_slots=None):
+               device=0, n_slots=None, symmetry="none"):
     """Plays network A (`weights_a`, the spec that `configs` build) against network B (`weights_b`, `spec_b` or A's spec)
     on one GPU.  Sharding a match over several GPUs is not supported.
 
@@ -127,6 +127,10 @@ def play_match(game_class, configs, weights_a, weights_b, n_games, spec_b=None, 
     * `iterations = (ia, ib)`: iteration limits of A's and B's searches (default `int(MCTS_iteration_limit * 1.5)` for both,
       as in self-play).  `max_actions` ends a game as a draw, counting the opening's plies.
     * `n_slots`: games resident on the GPU at once (default `games_per_gpu`, 4096).
+    * `symmetry`: how both networks evaluate a position (Engine.set_eval_symmetry): "none" (default, once as reached, the
+      reference's evaluation), "random" (one hashed board symmetry per request) or "ensemble" (the mean over all board
+      symmetries: a stronger, lower-variance evaluator at n times the network work - 8 for Gomoku / TicTacToe, 2 for
+      Connect4).  Only "none" keeps reference parity.
 
     Returns a dict: `wins` / `draws` / `losses` of A, `by_colour` (the same split by A moving first / second), `score`
     (W + D/2) / n, `elo` and its 95 % interval `elo_ci` (None at score 0 or 1), and `games`: per game `game_id`,
@@ -135,7 +139,7 @@ def play_match(game_class, configs, weights_a, weights_b, n_games, spec_b=None, 
     n_games = int(n_games)
     if n_games <= 0 or n_games % 2:
         raise ValueError("n_games must be a positive even number (games come in colour-swapped pairs), got %d" % n_games)
-    name, build_config, tc, explore, iterations, plies = _match_config(game_class, configs, 2, iterations, opening_plies)
+    name, build_config, tc, explore, iterations, plies = _match_config(game_class, configs, 2, iterations, opening_plies, symmetry)
     spec_a = net_spec_from_configs(name, build_config, configs[1])
     spec_b = spec_a if spec_b is None else spec_b
     book = opening_book(game_class, plies, seed)
@@ -289,7 +293,7 @@ def bradley_terry(points, games):
 
 
 def play_tournament(game_class, configs, weights, games_per_pair, specs=None, pairs=None, iterations=None,
-                    opening_plies=None, seed=0, device=0, n_slots=None):
+                    opening_plies=None, seed=0, device=0, n_slots=None, symmetry="none"):
     """Plays a tournament of K = len(weights) networks (2..8) on one GPU, every scheduled pair's games in one batch.
 
     * `pairs`: the schedule, by default the round robin (i, j), i < j (`round_robin`); a gauntlet is `gauntlet(K)`.
@@ -303,6 +307,7 @@ def play_tournament(game_class, configs, weights, games_per_pair, specs=None, pa
     * `iterations`: the K per-network iteration limits (default `int(MCTS_iteration_limit * 1.5)` for each).
     * `n_slots`: games resident on the GPU at once (default `games_per_gpu`, 4096); finished games are replaced by the
       next ones in id order, so pairs mix in the batch.
+    * `symmetry`: "none" (default, reference parity), "random" or "ensemble", for every network (as play_match).
 
     Returns a dict:
     * `pairs`: per scheduled pair `i`, `j`, wins / draws / losses of i, `by_colour` (i_first / i_second), `score` of i,
@@ -315,7 +320,7 @@ def play_tournament(game_class, configs, weights, games_per_pair, specs=None, pa
     K = len(weights)
     G_ = int(games_per_pair)
     pairs = check_schedule(K, G_, pairs)
-    name, build_config, tc, explore, iterations, plies = _match_config(game_class, configs, K, iterations, opening_plies)
+    name, build_config, tc, explore, iterations, plies = _match_config(game_class, configs, K, iterations, opening_plies, symmetry)
     default_spec = net_spec_from_configs(name, build_config, configs[1])
     specs = [default_spec] * K if specs is None else [default_spec if s is None else s for s in specs]
     if len(specs) != K:

@@ -501,6 +501,15 @@ static int launch_hash(gaz_engine *e, uint64_t salt, int logits) {
 }
 int gaz_internal_launch_select(gaz_engine *e) { return launch_select(e); }
 int gaz_internal_alloc(gaz_engine *e, void **p, size_t bytes) { return ealloc(e, (uint8_t **)p, bytes); }
+void gaz_internal_free(gaz_engine *e, void *p, size_t bytes) {
+    for (size_t i = 0; i < e->allocs.size(); i++)
+        if (e->allocs[i] == p) {
+            e->allocs.erase(e->allocs.begin() + (long)i);
+            e->bytes -= (int64_t)bytes;
+            dev_free(p);
+            return;
+        }
+}
 int gaz_internal_launch_expand(gaz_engine *e) { return launch_expand(e); }
 static int read_leaf_count(gaz_engine *e) {
     int32_t n = 0;
@@ -512,7 +521,7 @@ static int read_leaf_count(gaz_engine *e) {
 extern "C" {
 
 const char *gaz_last_error(void) { return g_err.c_str(); }
-int gaz_abi_version(void) { return 3; }
+int gaz_abi_version(void) { return 4; }
 
 int gaz_create(const gaz_config *cfg, gaz_engine **out) {
     if (!cfg || !out) return fail("null argument");
@@ -536,6 +545,7 @@ int gaz_create(const gaz_config *cfg, gaz_engine **out) {
     e->tree_net_max = 0;
     e->d_tree_net = nullptr;
     e->route = nullptr;
+    e->sym = nullptr;
     e->cache = nullptr;
     e->leaf_bound = 0;
     e->round_graph = nullptr; e->round_graph_chunks = 0; e->round_graph_warm = 0;
@@ -633,6 +643,7 @@ void gaz_destroy(gaz_engine *e) {
     for (void *p : e->allocs) dev_free(p);
     delete e->cache;
     delete e->route;
+    delete e->sym;
 #ifndef GAZ_EMUL
     if (e->ev0) { cudaEventDestroy(e->ev0); cudaEventDestroy(e->ev1); }
     cudaStreamDestroy(e->stream);
@@ -1180,6 +1191,8 @@ int gaz_eval_cache_enable(gaz_engine *e, int64_t entries, int shared_scope) {
     if (e->cache) return fail("the evaluation cache is already enabled");
     // the cache key does not include the network: a hit could hand one network's output to the other's trees
     if (e->n_nets > 1) return fail("the evaluation cache cannot be used with more than one attached network");
+    // a cache hit would return the symmetry drawn for the position's first evaluation
+    if (e->sym && e->sym->mode != GAZ_SYM_NONE) return fail("the evaluation cache cannot be used with symmetric evaluation");
     if (entries < 1024) return fail("evaluation cache: at least 1024 entries");
     const View &v = e->v;
     gaz_eval_cache *c = new gaz_eval_cache();

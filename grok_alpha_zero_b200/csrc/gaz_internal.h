@@ -60,7 +60,8 @@ struct gaz_engine {
     int n_nets;
     uint8_t *d_tree_net;   // [n_trees], allocated with the route buffers
     int tree_net_max;      // largest index in the uploaded table (host copy)
-    struct gaz_route *route; // packed per-network leaf lists, or null until two networks were attached
+    struct gaz_route *route; // packed per-network leaf lists, or null until two networks or a symmetry mode were set
+    struct gaz_sym *sym;     // symmetric evaluation (gaz_set_eval_symmetry), or null until it was first set
     struct gaz_eval_cache *cache; // evaluation cache or null
     int leaf_bound;      // host-side upper bound of outstanding leaf requests (0 = n_trees)
     // CUDA graph of one search round (select -> network -> expand), built by gaz_net.cu on first use
@@ -119,17 +120,29 @@ int gaz_internal_cache_fill(gaz_engine *e);
 
 // Several attached networks (a match, a tournament): every round the leaf list is partitioned by the network of each
 // leaf's tree, each network serves its own packed list and the outputs are scattered back to the leaf order (gaz_net.cu).
-// Lists 0..n_alloc-1 are allocated; attaching more networks later allocates the missing ones.
+// Lists 0..n_alloc-1 are allocated; attaching more networks later allocates the missing ones.  A packed list holds `cap`
+// rows: n_trees, or n_sym x n_trees while GAZ_SYM_ENSEMBLE evaluates every leaf under n_sym symmetries.
 struct gaz_route {
     int n_alloc;
+    size_t cap;
     int32_t *idx[GAZ_MAX_NETS];   // [n_trees]: leaf index of packed leaf m of network k
-    int32_t *count;               // [GAZ_MAX_NETS] device counts
-    int8_t *state[GAZ_MAX_NETS];  // [n_trees][S]
-    float *pol[GAZ_MAX_NETS];     // [n_trees][P]
-    float *val[GAZ_MAX_NETS];     // [n_trees]
+    int32_t *count;               // [GAZ_MAX_NETS] device counts (leaves)
+    int32_t *rows;                // [GAZ_MAX_NETS] device counts of packed rows (symmetric evaluation)
+    uint8_t *sym[GAZ_MAX_NETS];   // [n_trees]: GAZ_SYM_RANDOM's symmetry of packed leaf m of network k
+    int8_t *state[GAZ_MAX_NETS];  // [cap][S]
+    float *pol[GAZ_MAX_NETS];     // [cap][P]
+    float *val[GAZ_MAX_NETS];     // [cap]
 };
-// engine-owned device allocation (counted in gaz_bytes_allocated, freed with the engine)
+// Symmetric network evaluation (gaz_set_eval_symmetry): the tables live on the device as int16 (S, P <= 32767).
+struct gaz_sym {
+    int mode, n;                  // GAZ_SYM_*, rows of the tables
+    uint64_t seed;
+    int16_t *perm_state;          // [GAZ_MAX_SYM][S]
+    int16_t *perm_policy;         // [GAZ_MAX_SYM][P]
+};
+// engine-owned device allocation (counted in gaz_bytes_allocated, freed with the engine, or earlier by gaz_internal_free)
 int gaz_internal_alloc(gaz_engine *e, void **p, size_t bytes);
+void gaz_internal_free(gaz_engine *e, void *p, size_t bytes);
 
 int gaz_internal_launch_select(gaz_engine *e);
 int gaz_internal_launch_expand(gaz_engine *e);

@@ -360,6 +360,7 @@ __global__ void __launch_bounds__(128) policy_out_kernel(const int32_t *count, i
 }
 
 __global__ void set_count_kernel(int32_t *c, int v) { *c = v; }
+static constexpr int MAX_CHUNKS = 255;   // forward chunks per network and evaluation: 8 bits each in the round graph's key
 // leaves [offset, offset + max) of the request list form one forward chunk
 __global__ void chunk_count_kernel(const int32_t *total, int offset, int max, int32_t *out) {
     int c = *total - offset;
@@ -440,6 +441,111 @@ __global__ void __launch_bounds__(128) scatter_evals_kernel(int P, int K, const 
     if (lane == 0) value[leaf] = r.val[k][m];
 }
 
+// ---- symmetric evaluation (gaz_set_eval_symmetry): route -> pack (leaf, g) rows through perm_state[g] -> each network's
+// chunks -> map back through perm_policy[g] (and average the n_sym rows of a leaf in ENSEMBLE mode).
+__device__ __forceinline__ uint64_t sym_mix(uint64_t z) {   // splitmix64 finaliser
+    z ^= z >> 30; z *= 0xBF58476D1CE4E5B9ull;
+    z ^= z >> 27; z *= 0x94D049BB133111EBull;
+    return z ^ (z >> 31);
+}
+
+// GAZ_SYM_RANDOM's choice for one request, computed by a whole warp; oracle/sym_hash.py is the bit-identical twin.
+// acc = sum over the 8-byte little-endian words w_i of the state (zero-padded) of mix(w_i + (i + 1) * GOLD) mod 2^64;
+// h = mix(mix(mix(seed + GOLD) ^ key) ^ acc); g = (h >> 32) % n.
+__device__ __forceinline__ int sym_draw(const int8_t *st, int S, uint64_t seed, uint64_t key, int n, int lane) {
+    const uint64_t GOLD = 0x9E3779B97F4A7C15ull;
+    uint64_t acc = 0;
+    for (int w = lane; w * 8 < S; w += 32) {
+        uint64_t word = 0;
+        for (int b = 0; b < 8 && w * 8 + b < S; b++) word |= (uint64_t)(uint8_t)st[w * 8 + b] << (8 * b);
+        acc += sym_mix(word + (uint64_t)(w + 1) * GOLD);
+    }
+    for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
+    const uint64_t h = sym_mix(sym_mix(sym_mix(seed + GOLD) ^ key) ^ acc);
+    return (int)((h >> 32) % (uint64_t)n);
+}
+
+struct SymArgs {
+    const int16_t *perm;          // [n][S] (pack) or [n][P] (scatter)
+    int n, ensemble;              // table rows; 1 = every leaf gets n rows, 0 = one row of a drawn symmetry
+    uint64_t seed;
+    const uint64_t *tree_keys;    // per-tree keys or null (seed ^ tree)
+    float inv_n;                  // 1 / n (ENSEMBLE average)
+};
+
+// warp per packed row.  Packed leaf m of network k (route_leaves_kernel) becomes rows m*n .. m*n+n-1 of k's list (ENSEMBLE,
+// row m*n+g under symmetry g) or row m (RANDOM, under the drawn symmetry, kept in r.sym[k][m]); r.rows[k] = rows of k.
+__global__ void __launch_bounds__(256) sym_states_kernel(const gaz::LeafRec *leaves, const int8_t *leaf_state, int S, int K,
+                                                         const gaz_route r, const SymArgs a) {
+    extern __shared__ int16_t s_perm[];   // [n][S]
+    __shared__ int s_count[GAZ_MAX_NETS];
+    for (int i = threadIdx.x; i < a.n * S; i += blockDim.x) s_perm[i] = a.perm[i];
+    if (threadIdx.x < K) {
+        s_count[threadIdx.x] = r.count[threadIdx.x];
+        if (blockIdx.x == 0) r.rows[threadIdx.x] = r.count[threadIdx.x] * (a.ensemble ? a.n : 1);
+    }
+    __syncthreads();
+    int total = 0;
+    for (int k = 0; k < K; k++) total += s_count[k];
+    const int per = a.ensemble ? a.n : 1, lane = threadIdx.x & 31;
+    const int warps = (int)(gridDim.x * blockDim.x >> 5);
+    for (int row = (int)((blockIdx.x * blockDim.x + threadIdx.x) >> 5); row < total * per; row += warps) {
+        int k, m;
+        route_row(s_count, K, row / per, k, m);
+        const int leaf = r.idx[k][m];
+        const int8_t *src = leaf_state + (size_t)leaf * S;
+        int g = row % per;
+        if (!a.ensemble) {
+            const int tree = leaves[leaf].tree;
+            const uint64_t key = a.tree_keys ? a.tree_keys[tree] : a.seed ^ (uint64_t)(uint32_t)tree;
+            g = sym_draw(src, S, a.seed, key, a.n, lane);
+            if (lane == 0) r.sym[k][m] = (uint8_t)g;
+        }
+        int8_t *dst = r.state[k] + ((size_t)m * per + (a.ensemble ? g : 0)) * S;
+        const int16_t *pm = s_perm + g * S;
+        for (int j = lane; j < S; j += 32) dst[j] = src[pm[j]];
+    }
+}
+
+// warp per packed leaf: its row(s) go back to the leaf through perm_policy[g]; ENSEMBLE sums the n rows in g order in fp32
+// and multiplies by 1/n (policy entries and value alike)
+__global__ void __launch_bounds__(256) sym_scatter_kernel(int P, int K, const gaz_route r, const SymArgs a, float *policy,
+                                                          float *value) {
+    extern __shared__ int16_t s_perm[];   // [n][P]
+    __shared__ int s_count[GAZ_MAX_NETS];
+    for (int i = threadIdx.x; i < a.n * P; i += blockDim.x) s_perm[i] = a.perm[i];
+    if (threadIdx.x < K) s_count[threadIdx.x] = r.count[threadIdx.x];
+    __syncthreads();
+    int total = 0;
+    for (int k = 0; k < K; k++) total += s_count[k];
+    const int lane = threadIdx.x & 31, warps = (int)(gridDim.x * blockDim.x >> 5);
+    for (int row = (int)((blockIdx.x * blockDim.x + threadIdx.x) >> 5); row < total; row += warps) {
+        int k, m;
+        route_row(s_count, K, row, k, m);
+        const int leaf = r.idx[k][m];
+        float *dst = policy + (size_t)leaf * P;
+        if (!a.ensemble) {
+            const int g = r.sym[k][m];
+            const float *src = r.pol[k] + (size_t)m * P;
+            const int16_t *pm = s_perm + g * P;
+            for (int j = lane; j < P; j += 32) dst[j] = src[pm[j]];
+            if (lane == 0) value[leaf] = r.val[k][m];
+            continue;
+        }
+        const float *src = r.pol[k] + (size_t)m * a.n * P;
+        for (int j = lane; j < P; j += 32) {
+            float s = 0.0f;
+            for (int g = 0; g < a.n; g++) s += src[(size_t)g * P + s_perm[g * P + j]];
+            dst[j] = s * a.inv_n;
+        }
+        if (lane == 0) {
+            float s = 0.0f;
+            for (int g = 0; g < a.n; g++) s += r.val[k][(size_t)m * a.n + g];
+            value[leaf] = s * a.inv_n;
+        }
+    }
+}
+
 // ====================================================================== executor ==
 typedef CUresult (*PFN_encodeTiled)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *,
                                     const cuuint64_t *, const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave,
@@ -516,7 +622,9 @@ struct gaz_net {
     // I/O buffers for the host path (workspace)
     int8_t *d_states;
     int32_t *d_count;
-    int32_t *d_chunk_count; // [16] per-chunk leaf counts of an engine-driven forward
+    int32_t *d_chunk_count; // [chunk_cap] per-chunk leaf counts of an engine-driven forward
+    int chunk_cap;          // 16, or MAX_CHUNKS once an ENSEMBLE evaluation needed more (reserve_chunk_counts)
+    int32_t *d_chunk_count16; // the first 16-entry buffer after a growth (a round graph captured before may still read it)
     float *d_policy, *d_value;
     int logits_buf; // id of the flat buffer holding the policy logits
     // profiling of the tcgen05 conv launches
@@ -1007,6 +1115,8 @@ int gaz_net_create_shared(const gaz_net_desc *desc, gaz_net *share, gaz_net **ou
     rc |= walloc((void **)&n->d_states, (size_t)n->max_batch * n->H * n->W * n->Cin);
     rc |= alloc((void **)&n->d_count, 16);
     rc |= alloc((void **)&n->d_chunk_count, 16 * 4);
+    n->chunk_cap = 16;
+    n->d_chunk_count16 = nullptr;
     rc |= walloc((void **)&n->d_policy, (size_t)n->max_batch * n->P * 4);
     rc |= walloc((void **)&n->d_value, (size_t)n->max_batch * 4);
     if (rc != 0) { gaz_net_destroy(n); return -1; }
@@ -1515,6 +1625,7 @@ void gaz_net_destroy(gaz_net *n) {
     // bufs, d_act, d_xbf and the host-path staging belong to the workspace
     for (auto &op : n->ops) { if (op.d_se_b1) cudaFree(op.d_se_b1); if (op.d_wt) cudaFree(op.d_wt); if (op.d_stem_w) cudaFree(op.d_stem_w); if (op.d_stem_par) cudaFree(op.d_stem_par); if (op.d_frag) cudaFree(op.d_frag); if (op.d_hbias) cudaFree(op.d_hbias); if (op.d_frag0) cudaFree(op.d_frag0); }
     cudaFree(n->wf); cudaFree(n->wh); cudaFree(n->d_count); cudaFree(n->d_chunk_count);
+    if (n->d_chunk_count16) cudaFree(n->d_chunk_count16);
     if (n->ws && --n->ws->refs == 0) {
         for (void *p : n->ws->ptrs) cudaFree(p);
         delete n->ws;
@@ -1549,10 +1660,69 @@ static void drop_round_graph(gaz_engine *e) {
     e->attach_epoch++;
 }
 
+// Packed lists for the first K networks, each of at least `cap` rows (allocated on first use, grown when a symmetry mode
+// needs more rows; the round graph bakes in the pointers, so a regrowth drops it).
+static int route_reserve(gaz_engine *e, int K, size_t cap) {
+    const size_t NT = (size_t)e->v.n_trees, S = (size_t)e->v.ncell * e->v.C, P = (size_t)e->v.P;
+    if (!e->route) {
+        gaz_route r;
+        memset(&r, 0, sizeof r);
+        r.cap = NT;
+        if (gaz_internal_alloc(e, (void **)&r.count, GAZ_MAX_NETS * sizeof(int32_t)) != 0 ||
+            gaz_internal_alloc(e, (void **)&r.rows, GAZ_MAX_NETS * sizeof(int32_t)) != 0 ||
+            gaz_internal_alloc(e, (void **)&e->d_tree_net, NT) != 0)   // zero: every tree on network 0
+            return -1;
+        e->route = new gaz_route(r);
+    }
+    gaz_route &r = *e->route;
+    if (cap > r.cap) {   // new lists first: a failed allocation leaves the old ones in place
+        int8_t *st[GAZ_MAX_NETS] = {};
+        float *po[GAZ_MAX_NETS] = {}, *va[GAZ_MAX_NETS] = {};
+        auto undo = [&]() {
+            for (int k = 0; k < r.n_alloc; k++) {
+                if (st[k]) gaz_internal_free(e, st[k], cap * S);
+                if (po[k]) gaz_internal_free(e, po[k], cap * P * sizeof(float));
+                if (va[k]) gaz_internal_free(e, va[k], cap * sizeof(float));
+            }
+            return -1;
+        };
+        for (int k = 0; k < r.n_alloc; k++)
+            if (gaz_internal_alloc(e, (void **)&st[k], cap * S) != 0 || gaz_internal_alloc(e, (void **)&po[k], cap * P * sizeof(float)) != 0 ||
+                gaz_internal_alloc(e, (void **)&va[k], cap * sizeof(float)) != 0)
+                return undo();
+        CKN(cudaStreamSynchronize(e->stream));
+        drop_round_graph(e);
+        for (int k = 0; k < r.n_alloc; k++) {
+            gaz_internal_free(e, r.state[k], r.cap * S);
+            gaz_internal_free(e, r.pol[k], r.cap * P * sizeof(float));
+            gaz_internal_free(e, r.val[k], r.cap * sizeof(float));
+            r.state[k] = st[k]; r.pol[k] = po[k]; r.val[k] = va[k];
+        }
+        r.cap = cap;
+    }
+    for (int k = r.n_alloc; k < K; k++) {   // packed lists of the networks not seen before
+        if (gaz_internal_alloc(e, (void **)&r.idx[k], NT * sizeof(int32_t)) != 0 ||
+            gaz_internal_alloc(e, (void **)&r.sym[k], NT) != 0 ||
+            gaz_internal_alloc(e, (void **)&r.state[k], r.cap * S) != 0 ||
+            gaz_internal_alloc(e, (void **)&r.pol[k], r.cap * P * sizeof(float)) != 0 ||
+            gaz_internal_alloc(e, (void **)&r.val[k], r.cap * sizeof(float)) != 0)
+            return -1;
+        r.n_alloc = k + 1;
+    }
+    return 0;
+}
+
+static bool sym_on(const gaz_engine *e) { return e->sym && e->sym->mode != GAZ_SYM_NONE; }
+static int sym_rows_per_leaf(const gaz_engine *e) { return sym_on(e) && e->sym->mode == GAZ_SYM_ENSEMBLE ? e->sym->n : 1; }
+
 int gaz_attach_net(gaz_engine *e, gaz_net *n) {
     if (!e) return gaz_fail("null engine");
     if (n) {
         if (n->game != e->cfg.game) return gaz_fail("network game %d != engine game %d", n->game, e->cfg.game);
+    }
+    if (e->route && e->tree_net_max > 0) {   // the routed symmetric path reads the table: back to network 0
+        CKN(cudaMemsetAsync(e->d_tree_net, 0, (size_t)e->v.n_trees, e->stream));
+        e->tree_net_max = 0;
     }
     for (int k = 0; k < GAZ_MAX_NETS; k++) e->nets[k] = k == 0 ? n : nullptr;
     e->n_nets = n ? 1 : 0;
@@ -1574,24 +1744,8 @@ int gaz_attach_nets(gaz_engine *e, gaz_net *const *nets, int n_nets) {
         if (nets[k]->P != e->v.P)
             return gaz_fail("network %d has policy size %d (network 0: %d, engine: %d)", k, nets[k]->P, nets[0]->P, e->v.P);
     if (e->cache) return gaz_fail("%d networks cannot share the evaluation cache: its key does not include the network", n_nets);
-    const size_t NT = (size_t)e->v.n_trees, S = (size_t)e->v.ncell * e->v.C, P = (size_t)e->v.P;
-    if (!e->route) {
-        gaz_route r;
-        memset(&r, 0, sizeof r);
-        if (gaz_internal_alloc(e, (void **)&r.count, GAZ_MAX_NETS * sizeof(int32_t)) != 0 ||
-            gaz_internal_alloc(e, (void **)&e->d_tree_net, NT) != 0)   // zero: every tree on network 0
-            return -1;
-        e->route = new gaz_route(r);
-    }
-    for (int k = e->route->n_alloc; k < n_nets; k++) {   // packed lists of the networks not seen before
-        gaz_route &r = *e->route;
-        if (gaz_internal_alloc(e, (void **)&r.idx[k], NT * sizeof(int32_t)) != 0 ||
-            gaz_internal_alloc(e, (void **)&r.state[k], NT * S) != 0 ||
-            gaz_internal_alloc(e, (void **)&r.pol[k], NT * P * sizeof(float)) != 0 ||
-            gaz_internal_alloc(e, (void **)&r.val[k], NT * sizeof(float)) != 0)
-            return -1;
-        r.n_alloc = k + 1;
-    }
+    if (route_reserve(e, n_nets, (size_t)e->v.n_trees * sym_rows_per_leaf(e)) != 0) return -1;
+    const size_t NT = (size_t)e->v.n_trees;
     if (e->tree_net_max >= n_nets) {   // the table names a network that is no longer attached: back to network 0
         CKN(cudaMemsetAsync(e->d_tree_net, 0, NT, e->stream));
         e->tree_net_max = 0;
@@ -1616,12 +1770,68 @@ int gaz_set_tree_nets(gaz_engine *e, const uint8_t *tree_net) {
     return 0;
 }
 
-// forward chunks of network n over a packed request list of at most leaf_bound leaves (the count itself is on the device)
-static int forward_chunks(gaz_engine *e, gaz_net *n, const int32_t *total, const int8_t *states, float *pol, float *val) {
+int gaz_set_eval_symmetry(gaz_engine *e, int mode, int n_sym, const int32_t *perm_state, const int32_t *perm_policy,
+                          uint64_t seed) {
+    if (!e) return gaz_fail("null engine");
+    if (mode != GAZ_SYM_NONE && mode != GAZ_SYM_RANDOM && mode != GAZ_SYM_ENSEMBLE)
+        return gaz_fail("unknown symmetry mode %d (GAZ_SYM_NONE 0, GAZ_SYM_RANDOM 1, GAZ_SYM_ENSEMBLE 2)", mode);
+    if (mode == GAZ_SYM_NONE) {
+        if (sym_on(e)) { e->sym->mode = GAZ_SYM_NONE; drop_round_graph(e); }
+        return 0;
+    }
+    if (n_sym < 1 || n_sym > GAZ_MAX_SYM) return gaz_fail("n_sym = %d (1 to %d symmetries)", n_sym, GAZ_MAX_SYM);
+    if (!perm_state || !perm_policy) return gaz_fail("null symmetry table");
+    if (e->cache) return gaz_fail("symmetric evaluation cannot be used with the evaluation cache");
+    const int S = e->v.ncell * e->v.C, P = e->v.P;
+    std::vector<int16_t> ps((size_t)n_sym * S), pp((size_t)n_sym * P);
+    for (int t = 0; t < 2; t++) {
+        const int len = t == 0 ? S : P;
+        const int32_t *tab = t == 0 ? perm_state : perm_policy;
+        std::vector<char> seen((size_t)len);
+        for (int g = 0; g < n_sym; g++) {
+            std::fill(seen.begin(), seen.end(), 0);
+            for (int j = 0; j < len; j++) {
+                const int32_t x = tab[(size_t)g * len + j];
+                if (x < 0 || x >= len || seen[(size_t)x])
+                    return gaz_fail("%s row %d is not a permutation of 0..%d (entry %d = %d)", t == 0 ? "perm_state" : "perm_policy",
+                                    g, len - 1, j, (int)x);
+                seen[(size_t)x] = 1;
+                (t == 0 ? ps : pp)[(size_t)g * len + j] = (int16_t)x;
+            }
+        }
+    }
+    if (!e->sym) {
+        gaz_sym s;
+        memset(&s, 0, sizeof s);
+        if (gaz_internal_alloc(e, (void **)&s.perm_state, (size_t)GAZ_MAX_SYM * S * sizeof(int16_t)) != 0 ||
+            gaz_internal_alloc(e, (void **)&s.perm_policy, (size_t)GAZ_MAX_SYM * P * sizeof(int16_t)) != 0)
+            return -1;
+        e->sym = new gaz_sym(s);
+    }
+    const int K = e->n_nets > 1 ? e->n_nets : 1;
+    if (route_reserve(e, K, (size_t)e->v.n_trees * (mode == GAZ_SYM_ENSEMBLE ? n_sym : 1)) != 0) return -1;
+    if (e->tree_net_max >= K) {   // the table names a network that is no longer attached: back to network 0
+        CKN(cudaMemsetAsync(e->d_tree_net, 0, (size_t)e->v.n_trees, e->stream));
+        e->tree_net_max = 0;
+    }
+    // the tables are read from device memory: a captured round graph stays valid when only they change
+    CKN(cudaMemcpyAsync(e->sym->perm_state, ps.data(), ps.size() * sizeof(int16_t), cudaMemcpyHostToDevice, e->stream));
+    CKN(cudaMemcpyAsync(e->sym->perm_policy, pp.data(), pp.size() * sizeof(int16_t), cudaMemcpyHostToDevice, e->stream));
+    CKN(cudaStreamSynchronize(e->stream));
+    gaz_sym &s = *e->sym;
+    if (s.mode != mode || s.n != n_sym || s.seed != seed) drop_round_graph(e);
+    s.mode = mode; s.n = n_sym; s.seed = seed;
+    return 0;
+}
+
+// forward chunks of network n over a packed request list of at most rows_per_leaf x leaf_bound rows (the count itself is
+// on the device)
+static int forward_chunks(gaz_engine *e, gaz_net *n, int rows_per_leaf, const int32_t *total, const int8_t *states, float *pol,
+                          float *val) {
     const gaz::View &v = e->v;
-    const int bound = e->leaf_bound > 0 ? e->leaf_bound : v.n_trees;
+    const int bound = (e->leaf_bound > 0 ? e->leaf_bound : v.n_trees) * rows_per_leaf;
     const int chunks = (bound + n->max_batch - 1) / n->max_batch;
-    if (chunks > 16) return gaz_fail("leaf bound %d needs more than 16 chunks of %d", bound, n->max_batch);
+    if (chunks > n->chunk_cap) return gaz_fail("a bound of %d rows needs more than %d chunks of %d", bound, n->chunk_cap, n->max_batch);
     const size_t ss = (size_t)v.ncell * v.C;
     for (int ck = 0; ck < chunks; ck++) {
         const int off = ck * n->max_batch;
@@ -1635,6 +1845,25 @@ static int forward_chunks(gaz_engine *e, gaz_net *n, const int32_t *total, const
 // leaves (the host-side bound e->leaf_bound says how many chunks can be non-empty).
 static int engine_forward(gaz_engine *e) {
     const gaz::View &v = e->v;
+    if (sym_on(e)) {
+        // route (K = 1 too) -> pack (leaf, g) rows -> each network's chunks over rows_per_leaf x the leaf bound -> map back
+        const gaz_route &r = *e->route;
+        const gaz_sym &s = *e->sym;
+        const int K = e->n_nets, S = v.ncell * v.C, per = sym_rows_per_leaf(e);
+        const SymArgs pack{s.perm_state, s.n, per > 1, s.seed, v.tree_keys, 1.0f / (float)s.n};
+        const SymArgs back{s.perm_policy, s.n, per > 1, s.seed, v.tree_keys, 1.0f / (float)s.n};
+        auto blocks = [](size_t warps) { const size_t b = (warps + 7) / 8; return (unsigned)(b < 148 * 8 ? b : 148 * 8); };
+        route_leaves_kernel<<<1, 1024, 0, e->stream>>>(v.leaves, v.leaf_count, e->d_tree_net, K, r);
+        sym_states_kernel<<<blocks((size_t)v.n_trees * per), 256, (size_t)s.n * S * sizeof(int16_t), e->stream>>>(
+            v.leaves, v.leaf_state, S, K, r, pack);
+        CKN(cudaGetLastError());
+        for (int k = 0; k < K; k++)
+            if (forward_chunks(e, e->nets[k], per, r.rows + k, r.state[k], r.pol[k], r.val[k]) != 0) return -1;
+        sym_scatter_kernel<<<blocks((size_t)v.n_trees), 256, (size_t)s.n * v.P * sizeof(int16_t), e->stream>>>(
+            v.P, K, r, back, v.policy, v.value);
+        CKN(cudaGetLastError());
+        return 0;
+    }
     if (e->n_nets > 1) {
         // route -> each network's chunks in turn -> scatter.  Any packed list can hold every leaf, so each network gets the
         // chunks of the whole bound and a changed tree_net needs no new round graph.
@@ -1645,7 +1874,7 @@ static int engine_forward(gaz_engine *e) {
         route_states_kernel<<<rows, 128, 0, e->stream>>>(v.leaf_state, v.ncell * v.C, K, r);
         CKN(cudaGetLastError());
         for (int k = 0; k < K; k++)
-            if (forward_chunks(e, e->nets[k], r.count + k, r.state[k], r.pol[k], r.val[k]) != 0) return -1;
+            if (forward_chunks(e, e->nets[k], 1, r.count + k, r.state[k], r.pol[k], r.val[k]) != 0) return -1;
         scatter_evals_kernel<<<rows, 128, 0, e->stream>>>(v.P, K, r, v.policy, v.value);
         CKN(cudaGetLastError());
         return 0;
@@ -1656,13 +1885,35 @@ static int engine_forward(gaz_engine *e) {
     const int32_t *total = c ? c->miss_count : v.leaf_count;
     const int8_t *states = c ? c->packed_state : v.leaf_state;
     float *pol = c ? c->packed_pol : v.policy, *val = c ? c->packed_val : v.value;
-    if (forward_chunks(e, e->nets[0], total, states, pol, val) != 0) return -1;
+    if (forward_chunks(e, e->nets[0], 1, total, states, pol, val) != 0) return -1;
     if (c && gaz_internal_cache_fill(e) != 0) return -1;
+    return 0;
+}
+
+// Every network has 16 per-chunk counters, as many forward chunks as one evaluation of the leaf list takes; ENSEMBLE
+// evaluation serves n_sym rows per leaf and can take up to MAX_CHUNKS.  The larger buffer is allocated here, outside any
+// graph capture, on the first ENSEMBLE evaluation; the 16-entry one stays allocated with the network, since a round graph
+// captured before (by this or another engine) still reads it.
+static int reserve_chunk_counts(gaz_engine *e) {
+    if (sym_rows_per_leaf(e) == 1) return 0;
+    for (int k = 0; k < e->n_nets; k++) {
+        gaz_net *n = e->nets[k];
+        if (n->chunk_cap >= MAX_CHUNKS) continue;
+        int32_t *p = nullptr;
+        CKN(cudaMalloc((void **)&p, MAX_CHUNKS * 4));
+        CKN(cudaMemset(p, 0, MAX_CHUNKS * 4));
+        n->bytes += MAX_CHUNKS * 4;
+        n->d_chunk_count16 = n->d_chunk_count;
+        n->d_chunk_count = p;
+        n->chunk_cap = MAX_CHUNKS;
+        drop_round_graph(e);
+    }
     return 0;
 }
 
 int gaz_eval_net(gaz_engine *e) {
     if (!e || !e->n_nets) return gaz_fail("no network attached");
+    if (reserve_chunk_counts(e) != 0) return -1;
     return engine_forward(e);
 }
 
@@ -1677,9 +1928,10 @@ static int one_round_eager(gaz_engine *e) {
 // Every kernel reads its leaf count from device memory, so the graph does not depend on the data; it is rebuilt when
 // the number of forward chunks or the attached network set changes.  Disabled while conv launches are being event-timed.
 static int run_rounds(gaz_engine *e, int n_rounds) {
+    if (reserve_chunk_counts(e) != 0) return -1;
     bool profiling = false;
-    uint64_t chunks = 0;   // forward chunks of every attached network, 8 bits each (at most 16 chunks, 8 networks)
-    const int bound = e->leaf_bound > 0 ? e->leaf_bound : e->v.n_trees;
+    uint64_t chunks = 0;   // forward chunks of every attached network, 8 bits each (at most MAX_CHUNKS, 8 networks)
+    const int bound = (e->leaf_bound > 0 ? e->leaf_bound : e->v.n_trees) * sym_rows_per_leaf(e);
     for (int k = 0; k < e->n_nets; k++) {
         profiling = profiling || e->nets[k]->profile;
         chunks |= (uint64_t)((bound + e->nets[k]->max_batch - 1) / e->nets[k]->max_batch) << (8 * k);

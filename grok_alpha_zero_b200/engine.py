@@ -13,6 +13,7 @@ from . import _lib
 GAMES = {"tictactoe": 0, "connect4": 1, "gomoku": 2}
 DIMS = {"tictactoe": (3, 3, 2, 9), "connect4": (6, 7, 4, 7), "gomoku": (15, 15, 2, 225)}  # H, W, C, P
 TERM_NONE, TERM_DRAW, TERM_WIN = 0, 1, 2
+SYM_MODES = {"none": 0, "random": 1, "ensemble": 2}   # GAZ_SYM_* of include/gaz_net.h
 
 
 class EngineError(RuntimeError):
@@ -240,6 +241,20 @@ class Engine:
         """network index (< number of attached networks) of every tree, uint8 (n_trees,)"""
         t = np.ascontiguousarray(np.broadcast_to(np.asarray(tree_net), (self.n_trees,)), dtype=np.uint8)
         self._ck(self.lib.gaz_set_tree_nets(self._h, _p(t)))
+
+    def set_eval_symmetry(self, mode, seed=0):
+        """How the attached networks evaluate a request: "none" (default: once, as reached - the reference's behaviour),
+        "random" (under one board symmetry drawn from a hash of seed, tree key and position) or "ensemble" (the mean of
+        the outputs under all symmetries, mapped back; n times the network work).  Only "none" keeps reference parity.
+        Tables: games.eval_symmetries.  Cannot be combined with the evaluation cache."""
+        if mode not in SYM_MODES:
+            raise EngineError("unknown eval symmetry %r (one of %s)" % (mode, ", ".join(SYM_MODES)))
+        if SYM_MODES[mode] == 0:
+            self._ck(self.lib.gaz_set_eval_symmetry(self._h, 0, 0, None, None, 0))
+            return
+        from .games import eval_symmetries
+        ps, pp = eval_symmetries(self.game)
+        self._ck(self.lib.gaz_set_eval_symmetry(self._h, SYM_MODES[mode], ps.shape[0], _p(ps), _p(pp), int(seed) & (2**64 - 1)))
 
     def rounds_net(self, n, sync=True):
         fn = self.lib.gaz_rounds_net if sync else self.lib.gaz_rounds_net_async

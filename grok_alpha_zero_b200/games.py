@@ -326,6 +326,27 @@ class Connect4:
         return np.stack((board, np.fliplr(board))), np.stack((policy, np.fliplr(policy)))
 
 
+def eval_symmetries(name):
+    """Board symmetries for symmetric network evaluation (Engine.set_eval_symmetry), built from the board geometry:
+    the 8 dihedral maps in `_dihedral8`'s order for Gomoku and TicTacToe, the identity and the left-right column mirror
+    of all four planes for Connect4 (not Connect4.augment_sample, whose np.fliplr flips the rows: an upside-down board is
+    not a symmetry of the game).  Row 0 is the identity.  Returns (perm_state int32 (n, H*W*C), perm_policy int32 (n, P)):
+        state_g[j] = state[perm_state[g][j]]    (the transformed HWC input state, flattened)
+        p[a]       = q_g[perm_policy[g][a]]     (q_g = the network's policy row for state_g, p = the row mapped back)
+    so perm_policy[g][a] is the action that a takes to under symmetry g."""
+    H, W, C = {"gomoku": (15, 15, 2), "tictactoe": (3, 3, 2), "connect4": (6, 7, 4)}[name]
+    cells = np.arange(H * W).reshape(H, W)
+    maps = [cells, cells[:, ::-1]] if name == "connect4" else _dihedral8(cells)
+    perm_state, perm_policy = [], []
+    for m in maps:
+        src = np.ascontiguousarray(m).reshape(-1)                # cell c of the transformed board = cell src[c]
+        perm_state.append((src[:, None] * C + np.arange(C)).reshape(-1))
+        inv = np.empty_like(src)
+        inv[src] = np.arange(H * W)                              # original cell a sits at cell inv[a] of the transformed one
+        perm_policy.append(inv if name != "connect4" else inv[:W])
+    return np.array(perm_state, np.int32), np.array(perm_policy, np.int32)
+
+
 GAME_NAMES = {Gomoku: "gomoku", Connect4: "connect4", TicTacToe: "tictactoe"}
 
 

@@ -91,6 +91,25 @@ int gaz_attach_nets(gaz_engine *e, gaz_net *const *nets, int n_nets);
 /* tree_net: n_trees bytes, network index of every tree (< n_nets).  Stream-ordered upload; a captured round graph stays
  * valid (it reads the table from device memory). */
 int gaz_set_tree_nets(gaz_engine *e, const uint8_t *tree_net);
+
+/* Symmetric network evaluation.  GAZ_SYM_NONE (the default) evaluates every request once, in the orientation it was
+ * reached in, as the reference does.  GAZ_SYM_RANDOM evaluates each request under one board symmetry g drawn from a hash
+ * of (seed, the tree's key of gaz_set_tree_keys or seed ^ tree, the input-state bytes), so the draw does not depend on
+ * slots, batch layout, chunking or the number of GPUs (oracle/sym_hash.py is the hash's Python twin).  GAZ_SYM_ENSEMBLE
+ * evaluates it under all n_sym symmetries and averages the mapped-back outputs: fp32 sums in the order g = 0..n_sym-1,
+ * times 1/n_sym, for the policy row as the head returns it (probabilities, or logits for a linear head) and the value.
+ * Tables: n_sym rows of S = H*W*C (perm_state) and P (perm_policy) int32 entries, each row a permutation:
+ *   state_g[j] = state[perm_state[g][j]]        (the transformed input state)
+ *   p[a]       = q_g[perm_policy[g][a]]         (q_g = the network's policy row for state_g, p = the mapped-back row)
+ * grok_alpha_zero_b200.games.eval_symmetries builds them from the board geometry.  Applies to gaz_eval_net and
+ * gaz_rounds_net*, root evaluations included; not to gaz_put_evals or gaz_eval_hash.  Any mode but NONE routes the leaves
+ * like several networks do (also with one network) and cannot be combined with the evaluation cache.  Changing the mode,
+ * n_sym or seed re-captures the round graph; new tables of the same shape do not.  With GAZ_SYM_NONE the tables are
+ * ignored (may be NULL).  A refused call changes nothing. */
+enum { GAZ_SYM_NONE = 0, GAZ_SYM_RANDOM = 1, GAZ_SYM_ENSEMBLE = 2 };
+#define GAZ_MAX_SYM 8
+int gaz_set_eval_symmetry(gaz_engine *e, int mode, int n_sym, const int32_t *perm_state, const int32_t *perm_policy,
+                          uint64_t seed);
 int gaz_eval_net(gaz_engine *e);
 /* n_rounds x (select -> network -> expand), stream-ordered, no host sync inside; returns 0 */
 int gaz_rounds_net(gaz_engine *e, int n_rounds);
